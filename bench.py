@@ -2,6 +2,7 @@
 
   python bench.py [--gpus N] [--steps K] [--warmup W]                (N>1: launched under torchrun, one rank per GPU)
   python bench.py --impl reference [--gpus N] [--steps K] [--warmup W]
+  python bench.py [...] --dump-outputs DIR    (also writes the last timed step's outputs, see dump_outputs)
 
 Workload (BASELINE.json metric, configs[1]): 3-layer GraphSAGE (hidden 256, --use-pp, LayerNorm, dropout 0.5,
 lr 0.01, sampling rate 0.1) on the Reddit-shape synthetic power-law graph (232,965 nodes, ~114.6M edges, 602
@@ -135,6 +136,35 @@ def build_partition(shape: str, n_parts: int, rank: int, device):
     return part, stats
 
 
+DUMP_BYTES = 64 << 20            # --dump-outputs writes at most this much, all ranks together
+
+
+def dump_outputs(d: str, st, loss, rank: int, world: int) -> None:
+    """`--dump-outputs DIR`: what the last timed step computed, one `.npy` file per array, so that two builds run with
+    the same arguments can be compared output for output.  `loss` is the step's summed training loss on this rank,
+    `logits` this rank's inner nodes x classes, `param.<name>` the weights after the step's Adam update (identical on
+    every rank, so rank 0 writes them).  Logits larger than the budget are a fixed seeded sample of rows whose indices
+    go to `logits_rows`.  With several ranks, loss and logits carry a `.rank<r>` suffix."""
+    import numpy as np
+    os.makedirs(d, exist_ok=True)
+    sfx = f".rank{rank}" if world > 1 else ""
+    params = {f"param.{n}": p.detach().float() for n, p in st.model.named_parameters()}
+    out = {f"loss{sfx}": loss.detach().float().reshape(1)}
+    if rank == 0:
+        out.update(params)
+    logits = st.last_logits.detach().float()
+    n, c = logits.shape
+    budget = (DUMP_BYTES - sum(4 * p.numel() for p in params.values())) // world - 4
+    if 4 * n * c > budget:
+        keep = max(budget // (4 * c + 8), 0)
+        rows = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:keep].sort().values
+        out[f"logits_rows{sfx}"] = rows.double()
+        logits = logits[rows.to(logits.device)]
+    out[f"logits{sfx}"] = logits
+    for name, t in out.items():
+        np.save(os.path.join(d, name + ".npy"), t.cpu().numpy())
+
+
 # =====================================================================================================
 # our arm
 # =====================================================================================================
@@ -201,6 +231,7 @@ def run_ours(a):
 
     from bns_gcn_b200.module import dense as dense_mod
     dense_prof = []
+    last_loss = [None]                                   # what the most recent timed step returned
 
     def timed(step_fn, n_steps, profile_spmm):
         """n_steps of step_fn between barriers; device time by CUDA events, max over ranks."""
@@ -214,7 +245,7 @@ def run_ours(a):
         e0.record(torch.cuda.current_stream(dev))
         torch.cuda.nvtx.range_push("bns_timed")          # ncu --nvtx --nvtx-include "bns_timed/" lists the steps
         for _ in range(n_steps):
-            step_fn()
+            last_loss[0] = step_fn()
         torch.cuda.nvtx.range_pop()
         e1.record(torch.cuda.current_stream(dev))
         barrier()
@@ -228,11 +259,12 @@ def run_ours(a):
 
     def eager_step():
         nonlocal epoch
-        train.train_epoch(st, epoch)
+        loss = train.train_epoch(st, epoch)
         epoch += 1
         if world > 1:                                    # Comm(s) / Reduce(s) of EVERY eager epoch (train.py:415-418)
             comm_log.append(comm_timer.tot_time())
             reduce_log.append(ctx.reducer.last_reduce_seconds())
+        return loss
 
     # ---------------- eager pass: per-kernel CUDA events (roofline), Comm(s)/Reduce(s) -----------------------
     clocks = ClockSampler(local)
@@ -266,6 +298,8 @@ def run_ours(a):
             dev_ms, n_launch, _ = timed(eager_step, K, False)
     n0, n1 = 0, n_launch
     clk = clocks.stop() if rank == 0 else None
+    if a.dump_outputs:                                   # before the e2e pass below trains the model further
+        dump_outputs(a.dump_outputs, st, last_loss[0], rank, world)
     spmm_ms = sum(s.elapsed_time(e) for s, e, *_ in prof)
     spmm_alg = sum(p[2] for p in prof)
     spmm_gather = sum(4 * p[3] + 4 * p[4] * p[5] for p in prof)        # p[5]: entries actually gathered (estimate)
@@ -682,6 +716,8 @@ def main():
                          "(post-mortem of a hang on a box nobody can attach to); 0 = off")
     ap.add_argument("--strict", action="store_true", help="fail instead of falling back to eager when capture fails")
     ap.add_argument("--profile", default="", help="write a torch.profiler kernel table of 3 epochs (rank 0) to this file")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the loss, logits and weights of the last timed step to DIR/<name>.npy")
     # non-default workloads (the other BASELINE.json configs); the driver's contract run uses the defaults above
     ap.add_argument("--model", default=None, choices=["graphsage", "gcn", "gat"])
     ap.add_argument("--n-layers", type=int, default=None)

@@ -849,7 +849,7 @@ class GATRef(nn.Module):
             if i < self.n_layers - 1:
                 if self.use_norm:
                     h = self.norm[i](h)
-                h = F.relu(h)
+                h = _relu_on_active_set(h, rk, i)
         return h
 
 

@@ -52,6 +52,8 @@ def run_product(parts, args, device, n_epochs, selected_per_epoch=None, capture=
 
                 def pre(m, inp, i=i):
                     h = inp[1] if len(inp) > 1 else inp[0]
+                    if isinstance(h, tuple):             # GAT: (source rows, destination rows = the inner nodes)
+                        h = h[1]
                     cur_masks[i - 1] = (h[:n_in] > 0).detach().cpu()
                 hooks.append(layer.register_forward_pre_hook(pre))
         for e in range(n_epochs):
@@ -129,7 +131,7 @@ def run_parity_case(shape="tiny", n_parts=2, model="graphsage", sampling_rate=0.
     # CUDA path recording its active sets and the oracle on exactly those; accept the comparison only if every entry
     # that had to be switched sat within KINK_MARGIN of zero in the oracle's own forward.
     kink = None
-    if worst >= KINK_TRIGGER and model in ("graphsage", "gcn"):
+    if worst >= KINK_TRIGGER and model in ("graphsage", "gcn", "gat"):
         sel_in = selected if n_parts > 1 else None
         prod2 = run_product(parts, args, device, n_epochs, selected_per_epoch=sel_in, capture_masks=True)
         masks = [[prod2[r]["relu_masks"][e] for r in range(n_parts)] for e in range(n_epochs)]

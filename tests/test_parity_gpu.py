@@ -352,7 +352,11 @@ def test_cuda_gat_reproduces_the_reference_golden(built):
     processes, 2 heads, with dgl.nn.GATConv supplied as a DENSE masked-softmax restatement of DGL 0.9's layer.  The
     CUDA path (entry-list kernels; the 5-class output layer takes the op-by-op path), fed the index sets the reference
     drew, reproduces its stored halo features, head-averaged layer outputs, logits, reduced gradients and updated
-    weights within 1e-4 and its boundary sets exactly.  (Kept last in this file: new in round 2's final hours.)"""
+    weights within 1e-4 and its boundary sets exactly.
+
+    Epoch 3 of this run has one LayerNorm output about 1e-7 from zero (found by the oracle, which reproduces the golden to
+    1e-5), so the f32 forward on the GPU may take the other side of that ReLU kink; the fallback below is the one of the
+    eight-partition golden test."""
     import os
     from tests.harness import make_args, run_product, _relerr
     from bns_gcn_b200.data import make_graph, partition_graph
@@ -378,4 +382,13 @@ def test_cuda_gat_reproduces_the_reference_golden(built):
             errs[f"r{r}/param/{g['param_names'][k]}"] = _relerr(p, gp)
             errs[f"r{r}/grad/{g['param_names'][k]}"] = _relerr(o["grads"][k], gg)
     bad = {k: v for k, v in errs.items() if v >= TOL}
-    assert not bad, sorted(bad.items())
+    if bad:
+        # the oracle (tests/test_oracle_cpu.py pins it to this golden) on the active sets the CUDA forward took; accepted
+        # only if every switched entry sat within 1e-4 of zero in the oracle's own forward
+        from tests.harness import run_parity_case
+        res = run_parity_case(shape=cfg["shape"], n_parts=cfg["n_parts"], model=cfg["model"], sampling_rate=cfg["rate"],
+                              n_epochs=cfg["epochs"], n_layers=cfg["n_layers"], n_hidden=cfg["n_hidden"],
+                              heads=cfg["heads"], device="cuda:0", selected_per_epoch=sel)
+        assert res["kink"] is not None and res["kink"]["flips"] >= 1 and res["kink"]["max_abs_z"] < 1e-4, \
+            (sorted(bad.items()), res["kink"])
+        assert res["max_rel_err"] < TOL, ({k: v for k, v in res["detail"].items() if v >= TOL}, sorted(bad.items()))
