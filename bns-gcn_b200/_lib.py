@@ -13,7 +13,7 @@ from ctypes import POINTER, Structure, c_char_p, c_float, c_int, c_int32, c_int6
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "csrc", "libbnsgcn.so")
 
-ABI_VERSION = 2
+ABI_VERSION = 3
 P2P_HANDLE_BYTES = 64
 COMM_ID_BYTES = 128
 
@@ -67,8 +67,6 @@ SIGNATURES = {
     "bns_ln_relu_dropout_bwd_f32": (c_int, [c_void_p, c_int64, c_void_p, c_int64, c_int64, c_int64, c_void_p, c_void_p,
                                             c_void_p, c_void_p, c_float, c_float, c_uint64, c_uint64, c_void_p, c_void_p,
                                             c_int64, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
-    "bns_split_tf32_f32": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p]),
-    "bns_split_bf16x3_f32": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p]),
     "bns_dense_tn_3xtf32": (c_int, [c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_void_p, c_int64, c_void_p, c_void_p,
                                     c_int64, c_int64, c_int64, c_int64, c_void_p]),
     "bns_colsum_workspace_bytes": (c_size_t, [c_int64]),
@@ -91,13 +89,6 @@ SIGNATURES = {
     "bns_epoch_maps_update": (c_int, [POINTER(EpochMaps), c_void_p, c_size_t, c_void_p]),
     "bns_graph_compact_cols": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                        c_void_p]),
-    "bns_gat_forward_f32": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_int64, c_int32,
-                                    c_int32, c_void_p, c_void_p, c_float, c_float, c_uint64, c_uint64, c_void_p, c_void_p,
-                                    c_int64, c_void_p, c_void_p, c_void_p]),
-    "bns_gat_backward_f32": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_int64, c_int32,
-                                     c_int32, c_void_p, c_void_p, c_float, c_float, c_uint64, c_uint64, c_void_p, c_void_p,
-                                     c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
-                                     c_void_p]),
     "bns_gat_colsum_f32": (c_int, [c_void_p, c_void_p, c_int32, c_void_p, c_int64, c_void_p, c_void_p]),
     "bns_spmm_weighted_f32": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_int,
                                       c_void_p, c_int64, c_int, c_void_p, c_size_t, c_void_p]),

@@ -1479,84 +1479,6 @@ extern "C" int bns_colsum_f32(const float *X, int64_t ld, int64_t rows, int64_t 
 }
 
 // =================================================================================================
-// f32 -> 3 x bf16 split (dense layers, module/dense.py "bf16x3"): x = b0 + b1 + b2 to 24 bits of mantissa
-// =================================================================================================
-namespace {
-
-__device__ __forceinline__ unsigned short f32_to_bf16_rn(float f) {
-    unsigned int u = __float_as_uint(f);
-    u += 0x7fffu + ((u >> 16) & 1u);             // round to nearest even (inputs are finite)
-    return (unsigned short)(u >> 16);
-}
-__device__ __forceinline__ float bf16_to_f32(unsigned short h) { return __uint_as_float((unsigned int)h << 16); }
-
-__global__ void split_bf16x3_kernel(const float4 *__restrict__ x, int64_t n4, ushort4 *__restrict__ o0,
-                                    ushort4 *__restrict__ o1, ushort4 *__restrict__ o2) {
-    for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n4; i += (int64_t)gridDim.x * blockDim.x) {
-        const float4 v = x[i];
-        const float in[4] = {v.x, v.y, v.z, v.w};
-        unsigned short a[4], b[4], c[4];
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-            a[k] = f32_to_bf16_rn(in[k]);
-            const float r1 = in[k] - bf16_to_f32(a[k]);
-            b[k] = f32_to_bf16_rn(r1);
-            const float r2 = r1 - bf16_to_f32(b[k]);
-            c[k] = f32_to_bf16_rn(r2);
-        }
-        o0[i] = make_ushort4(a[0], a[1], a[2], a[3]);
-        o1[i] = make_ushort4(b[0], b[1], b[2], b[3]);
-        o2[i] = make_ushort4(c[0], c[1], c[2], c[3]);
-    }
-}
-
-}  // namespace
-
-namespace {
-// hi = x with the 13 low mantissa bits cleared after round-to-nearest (exactly representable in TF32, so neither a
-// truncating nor a rounding tensor-core path changes it), lo = x - hi (exact in f32)
-__global__ void split_tf32_kernel(const float4 *__restrict__ x, int64_t n4, float4 *__restrict__ hi, float4 *__restrict__ lo) {
-    for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n4; i += (int64_t)gridDim.x * blockDim.x) {
-        const float4 v = x[i];
-        float4 h, l;
-        h.x = __uint_as_float((__float_as_uint(v.x) + 0x1000u) & 0xffffe000u); l.x = v.x - h.x;
-        h.y = __uint_as_float((__float_as_uint(v.y) + 0x1000u) & 0xffffe000u); l.y = v.y - h.y;
-        h.z = __uint_as_float((__float_as_uint(v.z) + 0x1000u) & 0xffffe000u); l.z = v.z - h.z;
-        h.w = __uint_as_float((__float_as_uint(v.w) + 0x1000u) & 0xffffe000u); l.w = v.w - h.w;
-        hi[i] = h;
-        lo[i] = l;
-    }
-}
-}  // namespace
-
-extern "C" int bns_split_tf32_f32(const float *x, int64_t n, float *hi, float *lo, void *stream) {
-    BNS_REQUIRE(n >= 0 && n % 4 == 0, "bns_split_tf32_f32: element count must be a multiple of 4");
-    if (n == 0) return BNS_OK;
-    BNS_REQUIRE(x && hi && lo, "bns_split_tf32_f32: NULL pointer");
-    const int64_t n4 = n / 4;
-    int64_t want = (n4 + 255) / 256, cap = (int64_t)sm_count() * 16;
-    split_tf32_kernel<<<(unsigned)(want < cap ? want : cap), 256, 0, as_stream(stream)>>>(
-        reinterpret_cast<const float4 *>(x), n4, reinterpret_cast<float4 *>(hi), reinterpret_cast<float4 *>(lo));
-    ++g_launches;
-    BNS_CUDA(cudaGetLastError());
-    return BNS_OK;
-}
-
-extern "C" int bns_split_bf16x3_f32(const float *x, int64_t n, void *out0, void *out1, void *out2, void *stream) {
-    BNS_REQUIRE(n >= 0 && n % 4 == 0, "bns_split_bf16x3_f32: element count must be a multiple of 4");
-    if (n == 0) return BNS_OK;
-    BNS_REQUIRE(x && out0 && out1 && out2, "bns_split_bf16x3_f32: NULL pointer");
-    const int64_t n4 = n / 4;
-    int64_t want = (n4 + 255) / 256, cap = (int64_t)sm_count() * 16;
-    split_bf16x3_kernel<<<(unsigned)(want < cap ? want : cap), 256, 0, as_stream(stream)>>>(
-        reinterpret_cast<const float4 *>(x), n4, reinterpret_cast<ushort4 *>(out0), reinterpret_cast<ushort4 *>(out1),
-        reinterpret_cast<ushort4 *>(out2));
-    ++g_launches;
-    BNS_CUDA(cudaGetLastError());
-    return BNS_OK;
-}
-
-// =================================================================================================
 // halo slot map
 // =================================================================================================
 namespace {

@@ -7,9 +7,8 @@
 // 3xTF32 product  A*B ~= A_hi*B_hi + A_hi*B_lo + A_lo*B_hi  (hi = the TF32 part of x, lo = x - hi, exact in f32; the
 // dropped lo*lo term is ~2^-20 relative) with the operand split done INSIDE the pipeline: TMA lands the raw f32 tile
 // in shared memory, four "split" warps write lo beside it (element-wise, so the 128-byte swizzle pattern is
-// untouched; hi is the raw tile itself, see kTrunc below), then one thread issues the three MMAs per 8-wide k-step.
-// HBM/L2 see every operand once; the library-composed variant (module/dense.py "3xtf32") needs a split pass plus
-// three GEMMs.
+// untouched; hi is the raw tile itself, see gemm3x_kernel below), then one thread issues the three MMAs per 8-wide
+// k-step.  HBM/L2 see every operand once; composing the product from library GEMMs needs a split pass plus three GEMMs.
 //
 // A work item = one 128 x 128 output tile (x one slice of the contraction for the weight-gradient shape); persistent CTAs
 // of 320 threads walk the items:
@@ -133,20 +132,14 @@ __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&v)[32]) {
     asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
 }
 
-__device__ __forceinline__ float tf32_rna(float x) {
-    uint32_t u;
-    asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(u) : "f"(x));
-    return __uint_as_float(u);
-}
-
-// kTrunc: hi = x with the 13 low mantissa bits ignored BY THE TENSOR CORE (kind::tf32 reads the raw f32 words and drops
-// them -- verified on B200: same accuracy as the rounded variant), lo = x - trunc(x); saves the hi write-back, a third of
-// the split stage's shared-memory traffic.  Off (BNS_TC_TRUNC=0): hi = round-to-nearest TF32, written back in place.
+// The split: hi = x with the 13 low mantissa bits ignored BY THE TENSOR CORE (kind::tf32 reads the raw f32 words and
+// drops them), lo = x - trunc(x).  Measured on B200 as accurate as a round-to-nearest hi written back in place, and it
+// saves that write-back, a third of the split stage's shared-memory traffic.
 //
 // Persistent: gridDim.x = min(work items, SMs); a work item = (output tile, contraction slice).  All roles walk the same
 // item sequence; the shared-memory ring and its phases run on across items, and the accumulators are double-buffered in
 // TMEM (2 buffers x kAcc chains x 128 columns = all 512) so the epilogue of item i overlaps the main loop of item i+1.
-template <bool kMN, bool kTrunc>
+template <bool kMN>
 __global__ void __launch_bounds__(kThreadsTc, 1)
 gemm3x_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_b,
               float *__restrict__ C, int64_t ldc, int64_t split_stride, const float *__restrict__ bias,
@@ -269,20 +262,15 @@ gemm3x_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__
             for (int i = 0; i < nkb; ++i, ++g) {
                 const uint32_t s = g % kStages, ph = (g / kStages) & 1u;
                 mbar_wait(full_bar(s), ph);
-                float4 *raw = reinterpret_cast<float4 *>(base_ptr + s * STAGE_BYTES);
+                const float4 *raw = reinterpret_cast<const float4 *>(base_ptr + s * STAGE_BYTES);
                 float4 *lo = reinterpret_cast<float4 *>(base_ptr + s * STAGE_BYTES + RAW_BYTES);
 #pragma unroll 4
                 for (int j = 0; j < RAW_BYTES / 16 / kSplitThreads; ++j) {
                     const int idx = t + j * kSplitThreads;
                     const float4 x = raw[idx];
                     float4 h, l;
-                    if (kTrunc) {
-                        h.x = __uint_as_float(__float_as_uint(x.x) & 0xffffe000u); h.y = __uint_as_float(__float_as_uint(x.y) & 0xffffe000u);
-                        h.z = __uint_as_float(__float_as_uint(x.z) & 0xffffe000u); h.w = __uint_as_float(__float_as_uint(x.w) & 0xffffe000u);
-                    } else {
-                        h.x = tf32_rna(x.x); h.y = tf32_rna(x.y); h.z = tf32_rna(x.z); h.w = tf32_rna(x.w);
-                        raw[idx] = h;
-                    }
+                    h.x = __uint_as_float(__float_as_uint(x.x) & 0xffffe000u); h.y = __uint_as_float(__float_as_uint(x.y) & 0xffffe000u);
+                    h.z = __uint_as_float(__float_as_uint(x.z) & 0xffffe000u); h.w = __uint_as_float(__float_as_uint(x.w) & 0xffffe000u);
                     l.x = x.x - h.x; l.y = x.y - h.y; l.z = x.z - h.z; l.w = x.w - h.w;
                     lo[idx] = l;
                 }
@@ -358,266 +346,6 @@ gemm3x_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__
     }
 }
 
-// =====================================================================================================================
-// cta_group::2 variant: a CTA PAIR computes a 256 x 256 tile.  CTA c of the pair keeps A rows [128c, 128c + 128) and the
-// B rows (output columns) [128c, 128c + 128) of the pair tile -- the same 64 KB stage as the single-CTA kernel -- and the
-// leader issues  tcgen05.mma.cta_group::2  (M = 256, N = 256): each tensor core reads its own A tile and BOTH halves
-// of B, so the shared-memory operand reads per output halve (the single-CTA kernel is bound by exactly those reads).
-//   full[s]      local  : TMA -> this CTA's split warps
-//   split[s]     LEADER : 4 split warps of EACH CTA arrive (count 8; remote arrive through mapa)
-//   empty[s]     both   : the leader's tcgen05.commit multicasts to both CTAs -> each TMA producer
-//   acc_full     both   : multicast commit after the item's last k-block -> each CTA's epilogue warps
-//   acc_empty    LEADER : 4 epilogue warps of each CTA arrive (count 8) -> the MMA issuer may start the next item
-// TMEM: kAcc = 2 chains x 256 columns = all 512 columns, i.e. single-buffered: the epilogue is NOT overlapped here.
-// Enable with BNS_TC_PAIR=1 (module/dense.py picks it for N >= 192); validate with tools/check_dense_tc.py first.
-constexpr int BNP = 256;                        // pair tile width (and height: 2 x BM)
-
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-    uint32_t r;
-    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-    return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-    asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-    asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-// arrive on the barrier at the same shared-memory offset in CTA `cta` of the cluster
-__device__ __forceinline__ void mbar_arrive_cluster(uint32_t bar, uint32_t cta) {
-    asm volatile(
-        "{\n"
-        ".reg .b32 rem;\n"
-        "mapa.shared::cluster.u32 rem, %0, %1;\n"
-        "mbarrier.arrive.release.cluster.shared::cluster.b64 _, [rem];\n"
-        "}\n" ::"r"(bar), "r"(cta)
-        : "memory");
-}
-__device__ __forceinline__ void umma_tf32_pair(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc,
-                                               uint32_t accumulate) {
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "setp.ne.b32 p, %4, 0;\n"
-        "tcgen05.mma.cta_group::2.kind::tf32 [%0], %1, %2, %3, p;\n"
-        "}\n" ::"r"(d_tmem), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-__device__ __forceinline__ void umma_commit_pair(uint32_t bar) {
-    asm volatile(
-        "tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar),
-        "h"((uint16_t)3)
-        : "memory");
-}
-
-template <bool kMN>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreadsTc, 1)
-gemm3x_pair_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_b,
-                   float *__restrict__ C, int64_t ldc, int64_t split_stride, const float *__restrict__ bias,
-                   const float *__restrict__ addend, int64_t ldadd, const float *__restrict__ row_scale, int M, int N,
-                   int num_kb, int tiles_n, int tiles, int splits) {
-    extern __shared__ uint8_t smem_raw[];
-    const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const uint32_t cta = cluster_ctarank();
-    const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-    uint8_t *base_ptr = smem_raw + (base - smem_u32(smem_raw));
-    const uint32_t bars = base + kStages * STAGE_BYTES;
-    auto full_bar = [&](int s) { return bars + 8u * s; };
-    auto split_bar = [&](int s) { return bars + 8u * (kStages + s); };
-    auto empty_bar = [&](int s) { return bars + 8u * (2 * kStages + s); };
-    const uint32_t acc_full_bar = bars + 8u * (3 * kStages);
-    const uint32_t acc_empty_bar = bars + 8u * (3 * kStages + 1);
-    volatile uint32_t *tmem_slot = reinterpret_cast<volatile uint32_t *>(base_ptr + kStages * STAGE_BYTES + 8 * (3 * kStages + 2));
-
-    const int total_work = tiles * splits;
-    const int pair = blockIdx.x >> 1, n_pairs = gridDim.x >> 1;
-
-    if (warp == 0 && lane == 0) {
-        asm volatile("prefetch.tensormap [%0];" ::"l"(&map_a) : "memory");
-        asm volatile("prefetch.tensormap [%0];" ::"l"(&map_b) : "memory");
-        for (int s = 0; s < kStages; ++s) {
-            mbar_init(full_bar(s), 1);
-            mbar_init(split_bar(s), 2 * (kSplitThreads / 32));      // used on the leader only
-            mbar_init(empty_bar(s), 1);
-        }
-        mbar_init(acc_full_bar, 1);
-        mbar_init(acc_empty_bar, 2 * (kEpiThreads / 32));           // used on the leader only
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        asm volatile("fence.proxy.async;" ::: "memory");
-    }
-    if (warp == 1) {      // both CTAs, same warp id, same slot offset
-        asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32((const void *)tmem_slot)),
-                     "r"(512u)
-                     : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-    }
-    tc_fence_before();
-    cluster_sync_all();              // the peer's barriers exist before anybody arrives on them remotely
-    tc_fence_after();
-    const uint32_t tmem_base = *tmem_slot;
-
-#define BNS_TC_PAIR_ITEM(w)                                                   \
-    const int split_ = (w) / tiles, tile_ = (w) % tiles;                      \
-    const int m_t = tile_ / tiles_n, n_t = tile_ % tiles_n;                   \
-    const int kb0 = (int)(((int64_t)split_ * num_kb) / splits);               \
-    const int nkb = (int)(((int64_t)(split_ + 1) * num_kb) / splits) - kb0;
-
-    if (warp == 0) {
-        if (lane == 0) {
-            uint32_t g = 0;
-            for (int w = pair; w < total_work; w += n_pairs) {
-                BNS_TC_PAIR_ITEM(w)
-                const int m0 = m_t * 2 * BM + (int)cta * BM, n0 = n_t * BNP + (int)cta * BN;
-                for (int i = 0; i < nkb; ++i, ++g) {
-                    const uint32_t s = g % kStages, ph = (g / kStages) & 1u;
-                    mbar_wait(empty_bar(s), ph ^ 1u);
-                    mbar_expect_tx(full_bar(s), RAW_BYTES);
-                    const uint32_t a_dst = base + s * STAGE_BYTES, b_dst = a_dst + A_BYTES;
-                    const int kc = (kb0 + i) * BK;
-                    if (!kMN) {
-                        tma_load_2d(a_dst, &map_a, full_bar(s), kc, m0);
-                        tma_load_2d(b_dst, &map_b, full_bar(s), kc, n0);
-                    } else {
-#pragma unroll
-                        for (int b = 0; b < BM / 32; ++b) tma_load_2d(a_dst + b * MN_BOX_BYTES, &map_a, full_bar(s), m0 + 32 * b, kc);
-#pragma unroll
-                        for (int b = 0; b < BN / 32; ++b) tma_load_2d(b_dst + b * MN_BOX_BYTES, &map_b, full_bar(s), n0 + 32 * b, kc);
-                    }
-                }
-            }
-        }
-    } else if (warp == 1) {
-        if (lane == 0 && cta == 0) {
-            // instruction descriptor: D f32, A/B tf32, M = 256 (two CTAs), N = 256
-            const uint32_t idesc = (1u << 4) | (2u << 7) | (2u << 10) | ((kMN ? 1u : 0u) << 15) | ((kMN ? 1u : 0u) << 16) |
-                                   ((uint32_t)(BNP >> 3) << 17) | ((uint32_t)((2 * BM) >> 4) << 24);
-            const uint32_t lbo = kMN ? (uint32_t)MN_BOX_BYTES : 0u, sbo = kMN ? 512u : 1024u, lay = kMN ? 1u : 2u;
-            const uint32_t kstep = kMN ? 1024u : (uint32_t)(UMMA_K * 4);
-            uint32_t g = 0, it = 0;
-            for (int w = pair; w < total_work; w += n_pairs, ++it) {
-                BNS_TC_PAIR_ITEM(w)
-                (void)m_t; (void)n_t; (void)kb0;
-                mbar_wait(acc_empty_bar, (it & 1u) ^ 1u);
-                tc_fence_after();
-                for (int i = 0; i < nkb; ++i, ++g) {
-                    const uint32_t s = g % kStages, ph = (g / kStages) & 1u;
-                    mbar_wait(split_bar(s), ph);
-                    tc_fence_after();
-                    const uint32_t a_hi = base + s * STAGE_BYTES, b_hi = a_hi + A_BYTES;
-                    const uint32_t a_lo = a_hi + RAW_BYTES, b_lo = a_lo + A_BYTES;
-                    const uint32_t d = tmem_base + (uint32_t)(i % kAcc) * BNP;
-#pragma unroll
-                    for (int k = 0; k < BK / UMMA_K; ++k) {
-                        const uint64_t dah = smem_desc(a_hi + k * kstep, lbo, sbo, lay), dbh = smem_desc(b_hi + k * kstep, lbo, sbo, lay);
-                        const uint64_t dal = smem_desc(a_lo + k * kstep, lbo, sbo, lay), dbl = smem_desc(b_lo + k * kstep, lbo, sbo, lay);
-                        umma_tf32_pair(d, dal, dbh, idesc, (i >= kAcc || k != 0) ? 1u : 0u);
-                        umma_tf32_pair(d, dah, dbl, idesc, 1u);
-                        umma_tf32_pair(d, dah, dbh, idesc, 1u);
-                    }
-                    umma_commit_pair(empty_bar(s));
-                }
-                umma_commit_pair(acc_full_bar);
-            }
-        }
-    } else if (warp < 2 + kSplitThreads / 32) {
-        const int t = threadIdx.x - 64;
-        uint32_t g = 0;
-        for (int w = pair; w < total_work; w += n_pairs) {
-            BNS_TC_PAIR_ITEM(w)
-            (void)m_t; (void)n_t; (void)kb0;
-            for (int i = 0; i < nkb; ++i, ++g) {
-                const uint32_t s = g % kStages, ph = (g / kStages) & 1u;
-                mbar_wait(full_bar(s), ph);
-                const float4 *raw = reinterpret_cast<const float4 *>(base_ptr + s * STAGE_BYTES);
-                float4 *lo = reinterpret_cast<float4 *>(base_ptr + s * STAGE_BYTES + RAW_BYTES);
-#pragma unroll 4
-                for (int j = 0; j < RAW_BYTES / 16 / kSplitThreads; ++j) {
-                    const int idx = t + j * kSplitThreads;
-                    const float4 x = raw[idx];
-                    float4 l;
-                    l.x = x.x - __uint_as_float(__float_as_uint(x.x) & 0xffffe000u);
-                    l.y = x.y - __uint_as_float(__float_as_uint(x.y) & 0xffffe000u);
-                    l.z = x.z - __uint_as_float(__float_as_uint(x.z) & 0xffffe000u);
-                    l.w = x.w - __uint_as_float(__float_as_uint(x.w) & 0xffffe000u);
-                    lo[idx] = l;
-                }
-                asm volatile("fence.proxy.async;" ::: "memory");     // visible to the (leader-issued) MMA's reads of THIS CTA's smem
-                __syncwarp();
-                if (lane == 0) mbar_arrive_cluster(split_bar(s), 0);
-            }
-        }
-    } else {
-        const uint32_t q = warp & 3u;
-        uint32_t it = 0;
-        for (int w = pair; w < total_work; w += n_pairs, ++it) {
-            BNS_TC_PAIR_ITEM(w)
-            (void)kb0;
-            mbar_wait(acc_full_bar, it & 1u);
-            tc_fence_after();
-            const int nacc = nkb < kAcc ? nkb : kAcc;
-            const int row = m_t * 2 * BM + (int)cta * BM + (int)(32 * q + lane);
-            float *Cout = C + (int64_t)split_ * split_stride + (int64_t)row * ldc;
-            const float *Add = addend ? addend + (int64_t)row * ldadd : nullptr;
-            const float rsc = (row_scale && row < M) ? __ldg(row_scale + row) : 1.f;
-            const uint32_t tbase = tmem_base + ((32u * q) << 16);
-#pragma unroll 1
-            for (int c = 0; c < BNP / 32; ++c) {
-                uint32_t v[32];
-                tmem_ld32(tbase + (uint32_t)(c * 32), v);
-                for (int a = 1; a < nacc; ++a) {
-                    uint32_t u[32];
-                    tmem_ld32(tbase + (uint32_t)(a * BNP + c * 32), u);
-#pragma unroll
-                    for (int e = 0; e < 32; ++e) v[e] = __float_as_uint(__uint_as_float(v[e]) + __uint_as_float(u[e]));
-                }
-                const int col0 = n_t * BNP + c * 32;
-                if (row < M) {
-#pragma unroll
-                    for (int j = 0; j < 8; ++j) {
-                        const int col = col0 + 4 * j;
-                        if (col + 3 < N) {
-                            float4 o = make_float4(__uint_as_float(v[4 * j]), __uint_as_float(v[4 * j + 1]),
-                                                   __uint_as_float(v[4 * j + 2]), __uint_as_float(v[4 * j + 3]));
-                            if (bias) {
-                                const float4 bb = __ldg(reinterpret_cast<const float4 *>(bias + col));
-                                o.x += bb.x; o.y += bb.y; o.z += bb.z; o.w += bb.w;
-                            }
-                            if (Add) {
-                                const float4 aa = *reinterpret_cast<const float4 *>(Add + col);
-                                o.x += aa.x; o.y += aa.y; o.z += aa.z; o.w += aa.w;
-                            }
-                            if (row_scale) { o.x *= rsc; o.y *= rsc; o.z *= rsc; o.w *= rsc; }
-                            *reinterpret_cast<float4 *>(Cout + col) = o;
-                        } else {
-                            for (int e = 0; e < 4; ++e)
-                                if (col + e < N)
-                                    Cout[col + e] = (__uint_as_float(v[4 * j + e]) + (bias ? bias[col + e] : 0.f) + (Add ? Add[col + e] : 0.f)) * rsc;
-                        }
-                    }
-                }
-            }
-            tc_fence_before();
-            __syncwarp();
-            if (lane == 0) mbar_arrive_cluster(acc_empty_bar, 0);
-        }
-    }
-#undef BNS_TC_PAIR_ITEM
-
-    tc_fence_before();
-    cluster_sync_all();              // nobody frees TMEM / leaves while the peer's tensor core may still read its smem
-    if (warp == 1) {
-        __syncwarp();
-        asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
-    }
-}
-
-inline bool pair_mode() {
-    static int v = -1;
-    if (v < 0) {
-        const char *e = getenv("BNS_TC_PAIR");
-        v = (e && e[0] == '1') ? 1 : 0;
-    }
-    return v == 1;
-}
-
 // out[r, c] = sum_s ws[s][r, c]  in split order (deterministic); ws slices are contiguous [rows, cols]
 __global__ void splitk_reduce_kernel(const float4 *__restrict__ ws, int64_t slice4, int splits, int64_t cols4,
                                      float *__restrict__ out, int64_t ldo, int64_t total4) {
@@ -668,21 +396,12 @@ inline int make_map(CUtensorMap *m, const float *ptr, int64_t inner, int64_t row
 
 inline bool aligned16(const void *p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 
-inline bool trunc_mode() {
-    static int v = -1;
-    if (v < 0) {
-        const char *e = getenv("BNS_TC_TRUNC");
-        v = (e && e[0] == '0') ? 0 : 1;
-    }
-    return v == 1;
-}
-
-template <bool kMN, bool kTrunc>
+template <bool kMN>
 int configure() {
     static std::atomic<int> done[kMaxDevices];      // the attribute is per function AND per device
     const int dev = current_device();
     if (!done[dev].load(std::memory_order_acquire)) {
-        BNS_CUDA(cudaFuncSetAttribute(gemm3x_kernel<kMN, kTrunc>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
+        BNS_CUDA(cudaFuncSetAttribute(gemm3x_kernel<kMN>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
         done[dev].store(1, std::memory_order_release);
     }
     return BNS_OK;
@@ -705,37 +424,16 @@ extern "C" int bns_dense_tn_3xtf32(const float *A, int64_t lda, const float *B, 
     if (rc) return rc;
     rc = tc::make_map(&mb, B, K, N, ldb, tc::BK, tc::BN);
     if (rc) return rc;
-    const bool tr = tc::trunc_mode();
-    rc = tr ? tc::configure<false, true>() : tc::configure<false, false>();
+    rc = tc::configure<false>();
     if (rc) return rc;
     const int tiles_m = (int)((M + tc::BM - 1) / tc::BM), tiles_n = (int)((N + tc::BN - 1) / tc::BN);
     const int num_kb = (int)((K + tc::BK - 1) / tc::BK);
-    if (tc::pair_mode() && N >= 192) {      // DRAFT path (cta_group::2), see gemm3x_pair_kernel
-        static std::atomic<int> cfg_done[kMaxDevices];
-        const int dev = current_device();
-        if (!cfg_done[dev].load(std::memory_order_acquire)) {
-            BNS_CUDA(cudaFuncSetAttribute(tc::gemm3x_pair_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::SMEM_BYTES));
-            cfg_done[dev].store(1, std::memory_order_release);
-        }
-        const int ptm = (int)((M + 2 * tc::BM - 1) / (2 * tc::BM)), ptn = (int)((N + tc::BNP - 1) / tc::BNP);
-        const int ptiles = ptm * ptn, max_pairs = sm_count() / 2;
-        dim3 pgrid((unsigned)(2 * (ptiles < max_pairs ? ptiles : max_pairs)), 1, 1);
-        tc::gemm3x_pair_kernel<false><<<pgrid, tc::kThreadsTc, tc::SMEM_BYTES, as_stream(stream)>>>(
-            ma, mb, C, ldc, 0, bias, addend, ldadd, row_scale, (int)M, (int)N, num_kb, ptn, ptiles, 1);
-        ++g_launches;
-        BNS_CUDA(cudaGetLastError());
-        return BNS_OK;
-    }
     const int64_t tiles64 = tiles_m * (int64_t)tiles_n;
     BNS_REQUIRE(tiles64 < (1ll << 31), "bns_dense_tn_3xtf32: too many tiles");
     const int tiles = (int)tiles64;
     dim3 grid((unsigned)(tiles < sm_count() ? tiles : sm_count()), 1, 1);
-    if (tr)
-        tc::gemm3x_kernel<false, true><<<grid, tc::kThreadsTc, tc::SMEM_BYTES, as_stream(stream)>>>(ma, mb, C, ldc, 0, bias, addend, ldadd,
-                                                                                                   row_scale, (int)M, (int)N, num_kb, tiles_n, tiles, 1);
-    else
-        tc::gemm3x_kernel<false, false><<<grid, tc::kThreadsTc, tc::SMEM_BYTES, as_stream(stream)>>>(ma, mb, C, ldc, 0, bias, addend, ldadd,
-                                                                                                    row_scale, (int)M, (int)N, num_kb, tiles_n, tiles, 1);
+    tc::gemm3x_kernel<false><<<grid, tc::kThreadsTc, tc::SMEM_BYTES, as_stream(stream)>>>(ma, mb, C, ldc, 0, bias, addend, ldadd,
+                                                                                         row_scale, (int)M, (int)N, num_kb, tiles_n, tiles, 1);
     ++g_launches;
     BNS_CUDA(cudaGetLastError());
     return BNS_OK;
@@ -790,8 +488,7 @@ extern "C" int bns_dense_nt_3xtf32(const float *A, int64_t lda, const float *B, 
     if (rc) return rc;
     rc = tc::make_map(&mb, B, N2, R, ldb, 32, tc::BK, true);
     if (rc) return rc;
-    const bool tr = tc::trunc_mode();
-    rc = tr ? tc::configure<true, true>() : tc::configure<true, false>();
+    rc = tc::configure<true>();
     if (rc) return rc;
     const int tiles_m = (int)((N1 + tc::BM - 1) / tc::BM), tiles_n = (int)((N2 + tc::BN - 1) / tc::BN);
     const int num_kb = (int)((R + tc::BK - 1) / tc::BK);
@@ -802,12 +499,8 @@ extern "C" int bns_dense_nt_3xtf32(const float *A, int64_t lda, const float *B, 
     cudaStream_t st = as_stream(stream);
     float *w = splits == 1 ? C : static_cast<float *>(ws);
     const int64_t ldw = splits == 1 ? ldc : N2, slice = splits == 1 ? 0 : N1 * N2;
-    if (tr)
-        tc::gemm3x_kernel<true, true><<<grid, tc::kThreadsTc, tc::SMEM_BYTES, st>>>(ma, mb, w, ldw, slice, nullptr, nullptr, 0, nullptr,
-                                                                                    (int)N1, (int)N2, num_kb, tiles_n, tiles, splits);
-    else
-        tc::gemm3x_kernel<true, false><<<grid, tc::kThreadsTc, tc::SMEM_BYTES, st>>>(ma, mb, w, ldw, slice, nullptr, nullptr, 0, nullptr,
-                                                                                     (int)N1, (int)N2, num_kb, tiles_n, tiles, splits);
+    tc::gemm3x_kernel<true><<<grid, tc::kThreadsTc, tc::SMEM_BYTES, st>>>(ma, mb, w, ldw, slice, nullptr, nullptr, 0, nullptr,
+                                                                          (int)N1, (int)N2, num_kb, tiles_n, tiles, splits);
     if (splits == 1) {
         ++g_launches;
     } else {

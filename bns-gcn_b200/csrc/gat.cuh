@@ -1,28 +1,24 @@
 // gat.cuh -- GATConv's attention as kernels (included by bnsgcn.cu).  Reference: module/model.py:96-132 builds
 // dgl.nn.GATConv(in, out, heads, dropout, dropout); per layer DGL runs  e = leaky_relu(el_u + er_v)  (u_add_v),
 // a = edge_softmax(e), a = attn_drop(a), rst_v = sum_u a_uv ft_u  (u_mul_e + sum) and their autograd.  Round 1 did the
-// per-entry algebra with ~25 ATen launches over [nnz, heads] temporaries and one SpMM launch per head.  Here, two forms
-// of the same algebra (same Philox mask, tests compare them):
+// per-entry algebra with ~25 ATen launches over [nnz, heads] temporaries and one SpMM launch per head.  Here the
+// algebra is staged: scalar row walks for the softmax, the tuned SpMM / SDDMM kernels for everything F-wide.
 //
-// (A) staged -- what graph.GatAttention runs (profiles/gat_r02.md: 2-3x faster on low-degree graphs)
 //   gat_proj_kernel / gat_proj_bwd_kernel   el = <ft, attn_l>, er = <ft, attn_r> per head and their backward
 //   gat_scores_kernel        one warp per destination row, scalars only: score -> online max / sum -> probability P and
 //                            dropped attention a' per entry (a' of the halo entries also at their compacted positions)
 //   (rst = A' ft is the weighted SpMM per head: bns_spmm_weighted_f32 + bns_spmm_compact_f32;
 //    d a' = <d rst_v, ft_u> is bns_sddmm_dot_f32)
 //   gat_softmax_bwd_kernel   one warp per destination row, scalars only: d a' -> d e per entry (in place), d er_v
-//
-// (B) one launch per direction (BNS_GAT_ROWWALK=1)
-//   gat_fwd_kernel     one warp per destination row, all heads: score -> max -> sum -> probability (stored per entry for
-//                      the backward) -> Philox dropout -> weighted accumulation of the gathered ft rows
-//   gat_bwd_kernel     one warp per destination row: d a = <d rst_v, ft_u> (SDDMM) -> softmax / leaky-relu backward ->
-//                      d e per entry, d er_v; writes the dropped attention a' for the transposed SpMM
-//
-// both:
-//   gat_colsum_kernel  d el_u = sum over the entries of column u of d e (walks the static transposes through their
-//                      entry permutation: deterministic, no atomics)
+//   gat_colsum_kernel        d el_u = sum over the entries of column u of d e (walks the static transposes through their
+//                            entry permutation: deterministic, no atomics)
 //   (d ft = A'^T d rst is the weighted transposed SpMM: spmm_kernel with per-entry weights looked up through the
 //    permutation, bns_spmm_weighted_f32)
+//
+// A fused form -- one warp per destination row doing scores, softmax, dropout and the weighted accumulation of the
+// gathered ft rows in one launch per direction -- keeps one row's dependent loads in flight per warp; on a low-degree
+// graph (Yelp shape, ~20 entries per row) that is a latency chain per row, and it measured 3x slower than the staged
+// form, whose SpMM keeps 8 gathers in flight per lane (profiles/gat_r02.md).
 //
 // The row's entries are the inner ones (a_in) followed by this epoch's SAMPLED halo ones (a_out after
 // bns_graph_compact_cols: chunk-local compaction, so a row is walked chunk by chunk through row_chunk).
@@ -39,16 +35,12 @@ struct GatGraph {
 
 struct GatArgs {
     GatGraph g;
-    const float *ft; int64_t ldft; int32_t H, Fo;
+    int32_t H;
     const float *el, *er;                                                  // [n_u, H], [n_rows, H]
     float slope, p_drop, keep_scale;
     uint64_t seed, offset; const uint64_t *offset_dev;
-    // forward
-    float *rst; int64_t ldr;
     float *P_in, *P_out;                                                   // [nnz, H] at the ORIGINAL entry positions
-    // backward
-    const float *d_rst; int64_t ldd;
-    float *dE_in, *dE_out, *A_in, *A_out, *d_er;
+    float *dE_in, *dE_out, *d_er;                                          // backward
 };
 
 __device__ __forceinline__ float leaky(float x, float slope) { return x > 0.f ? x : x * slope; }
@@ -82,271 +74,6 @@ __device__ __forceinline__ bool gat_keep(uint64_t seed, uint64_t offset, int64_t
             }                                                                                        \
         }                                                                                            \
     }
-
-template <int NV>
-__global__ void __launch_bounds__(kThreads) gat_fwd_kernel(GatArgs a, int64_t nnz_in) {
-    __shared__ int32_t s_u[kWarps][32];
-    __shared__ float s_w[kWarps][32][kGatMaxHeads];
-    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-    const int64_t warps_total = (int64_t)gridDim.x * kWarps;
-    const uint64_t offset = a.offset + (a.offset_dev ? *a.offset_dev : 0ull);
-    const int H = a.H, F = a.H * a.Fo;
-    int hd[NV];                                   // head that owns each float4 column group of this lane
-#pragma unroll
-    for (int t = 0; t < NV; ++t) {
-        const int c = (lane + 32 * t) * 4;
-        hd[t] = c < F ? c / a.Fo : 0;
-    }
-    for (int64_t v = (int64_t)blockIdx.x * kWarps + w; v < a.g.n_rows; v += warps_total) {
-        float erv[kGatMaxHeads], m[kGatMaxHeads], l[kGatMaxHeads];
-#pragma unroll
-        for (int h = 0; h < kGatMaxHeads; ++h) {
-            erv[h] = h < H ? a.er[v * H + h] : 0.f;
-            m[h] = -INFINITY;
-            l[h] = 0.f;
-        }
-        // walk 1: per-lane online (max, sum of exp) of the scores, then one cross-lane combine per head
-        BNS_GAT_FOR_EACH_ENTRY({
-            (void)pos; (void)halo;
-_Pragma("unroll")
-            for (int h = 0; h < kGatMaxHeads; ++h)
-                if (h < H) {
-                    const float sc = leaky(a.el[(int64_t)u * H + h] + erv[h], a.slope);
-                    if (sc > m[h]) { l[h] = l[h] * expf(m[h] - sc) + 1.f; m[h] = sc; }
-                    else l[h] += expf(sc - m[h]);
-                }
-        })
-#pragma unroll
-        for (int h = 0; h < kGatMaxHeads; ++h) {
-            float mt = m[h];
-#pragma unroll
-            for (int o = 16; o > 0; o >>= 1) mt = fmaxf(mt, __shfl_xor_sync(0xffffffffu, mt, o));
-            l[h] = warp_sum(m[h] == -INFINITY ? 0.f : l[h] * expf(m[h] - mt));
-            m[h] = mt;
-        }
-        // walk 2: probabilities (stored), dropout, weighted accumulation -- 32 entries at a time through shared memory
-        float4 acc[NV];
-#pragma unroll
-        for (int t = 0; t < NV; ++t) acc[t] = make_float4(0.f, 0.f, 0.f, 0.f);
-        constexpr int U = NV <= 2 ? 4 : (NV == 4 ? 2 : 1);        // entries whose row gathers are in flight together
-        auto consume = [&](int cnt) {
-            __syncwarp();
-            int jj = 0;
-            for (; jj + U <= cnt; jj += U) {
-                float4 x[U][NV];
-#pragma unroll
-                for (int q = 0; q < U; ++q) {
-                    const float *fr = a.ft + (int64_t)s_u[w][jj + q] * a.ldft;
-#pragma unroll
-                    for (int t = 0; t < NV; ++t) {
-                        const int c = (lane + 32 * t) * 4;
-                        x[q][t] = c < F ? __ldg(reinterpret_cast<const float4 *>(fr + c)) : make_float4(0.f, 0.f, 0.f, 0.f);
-                    }
-                }
-#pragma unroll
-                for (int q = 0; q < U; ++q)
-#pragma unroll
-                    for (int t = 0; t < NV; ++t) {
-                        const float wt = s_w[w][jj + q][hd[t]];
-                        acc[t].x = fmaf(x[q][t].x, wt, acc[t].x); acc[t].y = fmaf(x[q][t].y, wt, acc[t].y);
-                        acc[t].z = fmaf(x[q][t].z, wt, acc[t].z); acc[t].w = fmaf(x[q][t].w, wt, acc[t].w);
-                    }
-            }
-            for (; jj < cnt; ++jj) {
-                const float *fr = a.ft + (int64_t)s_u[w][jj] * a.ldft;
-#pragma unroll
-                for (int t = 0; t < NV; ++t) {
-                    const int c = (lane + 32 * t) * 4;
-                    if (c < F) {
-                        const float wt = s_w[w][jj][hd[t]];
-                        const float4 x = __ldg(reinterpret_cast<const float4 *>(fr + c));
-                        acc[t].x = fmaf(x.x, wt, acc[t].x); acc[t].y = fmaf(x.y, wt, acc[t].y);
-                        acc[t].z = fmaf(x.z, wt, acc[t].z); acc[t].w = fmaf(x.w, wt, acc[t].w);
-                    }
-                }
-            }
-            __syncwarp();
-        };
-        auto stage = [&](bool valid, int32_t u, int64_t pos, bool halo) {
-            if (valid) {
-                s_u[w][lane] = u;
-                float *P = (halo ? a.P_out : a.P_in) + pos * H;
-                const int64_t gid = halo ? nnz_in + pos : pos;
-#pragma unroll
-                for (int h = 0; h < kGatMaxHeads; ++h)
-                    if (h < H) {
-                        const float p = expf(leaky(a.el[(int64_t)u * H + h] + erv[h], a.slope) - m[h]) / l[h];
-                        P[h] = p;
-                        float wt = p;
-                        if (a.p_drop > 0.f) wt = gat_keep(a.seed, offset, gid, h, a.p_drop) ? p * a.keep_scale : 0.f;
-                        s_w[w][lane][h] = wt;
-                    }
-            }
-        };
-        {
-            const int64_t b = a.g.in_ptr[v], e = a.g.in_ptr[v + 1];
-            for (int64_t k0 = b; k0 < e; k0 += 32) {
-                const int64_t k = k0 + lane;
-                const bool valid = k < e;
-                stage(valid, valid ? a.g.in_idx[k] : 0, k, false);
-                consume((int)((e - k0) < 32 ? (e - k0) : 32));
-            }
-        }
-        if (a.g.cidx) {
-            for (int32_t c = a.g.out_row_chunk[v]; c < a.g.out_row_chunk[v + 1]; ++c) {
-                const int64_t s0 = a.g.out_chunk_start[c];
-                const int32_t cnt = a.g.chunk_cnt[c];
-                for (int32_t j0 = 0; j0 < cnt; j0 += 32) {
-                    const int32_t j = j0 + lane;
-                    const bool valid = j < cnt;
-                    stage(valid, valid ? (int32_t)a.g.x_halo_base + a.g.cidx[s0 + j] : 0, valid ? a.g.cpos[s0 + j] : 0, true);
-                    consume((cnt - j0) < 32 ? (cnt - j0) : 32);
-                }
-            }
-        }
-        float *out = a.rst + v * a.ldr;
-#pragma unroll
-        for (int t = 0; t < NV; ++t) {
-            const int c = (lane + 32 * t) * 4;
-            if (c < F) *reinterpret_cast<float4 *>(out + c) = acc[t];
-        }
-    }
-}
-
-template <int NV>
-__global__ void __launch_bounds__(kThreads) gat_bwd_kernel(GatArgs a, int64_t nnz_in) {
-    __shared__ int32_t s_u[kWarps][32];
-    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-    const int64_t warps_total = (int64_t)gridDim.x * kWarps;
-    const uint64_t offset = a.offset + (a.offset_dev ? *a.offset_dev : 0ull);
-    const int H = a.H, F = a.H * a.Fo;
-    int hd[NV];
-#pragma unroll
-    for (int t = 0; t < NV; ++t) {
-        const int c = (lane + 32 * t) * 4;
-        hd[t] = c < F ? c / a.Fo : 0;
-    }
-    for (int64_t v = (int64_t)blockIdx.x * kWarps + w; v < a.g.n_rows; v += warps_total) {
-        float erv[kGatMaxHeads], rowdot[kGatMaxHeads], der[kGatMaxHeads];
-#pragma unroll
-        for (int h = 0; h < kGatMaxHeads; ++h) {
-            erv[h] = h < H ? a.er[v * H + h] : 0.f;
-            rowdot[h] = 0.f;
-            der[h] = 0.f;
-        }
-        float4 dv[NV];
-#pragma unroll
-        for (int t = 0; t < NV; ++t) {
-            const int c = (lane + 32 * t) * 4;
-            dv[t] = c < F ? *reinterpret_cast<const float4 *>(a.d_rst + v * a.ldd + c) : make_float4(0.f, 0.f, 0.f, 0.f);
-        }
-        // pass A: d a'_uv = <d rst_v, ft_u> per head (all lanes per entry), d p = mask / (1 - q) * d a'; parked in dE
-        auto dots = [&](int cnt, bool valid, int64_t pos, bool halo) {
-            __syncwarp();
-            float mine[kGatMaxHeads];
-#pragma unroll
-            for (int h = 0; h < kGatMaxHeads; ++h) mine[h] = 0.f;
-            constexpr int U = NV <= 2 ? 4 : (NV == 4 ? 2 : 1);
-            for (int j0 = 0; j0 < cnt; j0 += U) {
-                float4 x[U][NV];
-#pragma unroll
-                for (int q = 0; q < U; ++q) {
-                    const int jj = j0 + q < cnt ? j0 + q : cnt - 1;           // (a repeated last row: its dot is discarded)
-                    const float *fr = a.ft + (int64_t)s_u[w][jj] * a.ldft;
-#pragma unroll
-                    for (int t = 0; t < NV; ++t) {
-                        const int c = (lane + 32 * t) * 4;
-                        x[q][t] = c < F ? __ldg(reinterpret_cast<const float4 *>(fr + c)) : make_float4(0.f, 0.f, 0.f, 0.f);
-                    }
-                }
-#pragma unroll
-                for (int q = 0; q < U; ++q) {
-                    float part[kGatMaxHeads];
-#pragma unroll
-                    for (int h = 0; h < kGatMaxHeads; ++h) part[h] = 0.f;
-#pragma unroll
-                    for (int t = 0; t < NV; ++t) {
-                        const float d = (dv[t].x * x[q][t].x + dv[t].y * x[q][t].y) + (dv[t].z * x[q][t].z + dv[t].w * x[q][t].w);
-#pragma unroll
-                        for (int h = 0; h < kGatMaxHeads; ++h)
-                            if (h == hd[t]) part[h] += d;
-                    }
-#pragma unroll
-                    for (int h = 0; h < kGatMaxHeads; ++h)
-                        if (h < H) {
-                            const float tot = warp_sum(part[h]);
-                            if (lane == j0 + q) mine[h] = tot;
-                        }
-                }
-            }
-            if (valid) {
-                const float *P = (halo ? a.P_out : a.P_in) + pos * H;
-                float *dE = (halo ? a.dE_out : a.dE_in) + pos * H;
-                float *A = halo ? a.A_out : a.A_in;
-                const int64_t gid = halo ? nnz_in + pos : pos;
-#pragma unroll
-                for (int h = 0; h < kGatMaxHeads; ++h)
-                    if (h < H) {
-                        float ms = 1.f;
-                        if (a.p_drop > 0.f) ms = gat_keep(a.seed, offset, gid, h, a.p_drop) ? a.keep_scale : 0.f;
-                        const float dp = mine[h] * ms;
-                        dE[h] = dp;
-                        rowdot[h] += P[h] * dp;
-                        if (A) A[pos * H + h] = P[h] * ms;
-                    }
-            }
-            __syncwarp();
-        };
-        {
-            const int64_t b = a.g.in_ptr[v], e = a.g.in_ptr[v + 1];
-            for (int64_t k0 = b; k0 < e; k0 += 32) {
-                const int64_t k = k0 + lane;
-                const bool valid = k < e;
-                if (valid) s_u[w][lane] = a.g.in_idx[k];
-                dots((int)((e - k0) < 32 ? (e - k0) : 32), valid, k, false);
-            }
-        }
-        if (a.g.cidx) {
-            for (int32_t c = a.g.out_row_chunk[v]; c < a.g.out_row_chunk[v + 1]; ++c) {
-                const int64_t s0 = a.g.out_chunk_start[c];
-                const int32_t cnt = a.g.chunk_cnt[c];
-                for (int32_t j0 = 0; j0 < cnt; j0 += 32) {
-                    const int32_t j = j0 + lane;
-                    const bool valid = j < cnt;
-                    if (valid) s_u[w][lane] = (int32_t)a.g.x_halo_base + a.g.cidx[s0 + j];
-                    dots((cnt - j0) < 32 ? (cnt - j0) : 32, valid, valid ? a.g.cpos[s0 + j] : 0, true);
-                }
-            }
-        }
-#pragma unroll
-        for (int h = 0; h < kGatMaxHeads; ++h) rowdot[h] = warp_sum(rowdot[h]);
-        // pass B: softmax backward, leaky-relu backward: d e per entry, d er_v
-        BNS_GAT_FOR_EACH_ENTRY({
-            const float *P = (halo ? a.P_out : a.P_in) + pos * H;
-            float *dE = (halo ? a.dE_out : a.dE_in) + pos * H;
-_Pragma("unroll")
-            for (int h = 0; h < kGatMaxHeads; ++h)
-                if (h < H) {
-                    const float ds = P[h] * (dE[h] - rowdot[h]);
-                    const float raw = a.el[(int64_t)u * H + h] + erv[h];
-                    const float de = raw > 0.f ? ds : ds * a.slope;
-                    dE[h] = de;
-                    der[h] += de;
-                }
-        })
-#pragma unroll
-        for (int h = 0; h < kGatMaxHeads; ++h) {
-            der[h] = warp_sum(der[h]);
-            if (lane == 0 && h < H) a.d_er[v * H + h] = der[h];
-        }
-    }
-}
-
-// ---- the decomposed form: scalar row walks + the tuned SpMM / SDDMM kernels for everything F-wide --------------------
-// The fused row-walk kernels above keep ONE row's dependent loads in flight per warp; on a low-degree graph (Yelp shape,
-// ~20 entries per row) that is a latency chain per row and 2-9 ms per launch (profiles/gat_r02.md).  The same algebra
-// as: scores kernel (scalars only) -> weighted SpMM (spmm_kernel, 8 gathers in flight per lane) in forward, and
-// SDDMM -> softmax/leaky backward (scalars only) -> column sums -> weighted transposed SpMM in backward.
 
 // P (probabilities, original positions), W (dropped attention a' = p * mask / (1 - q), original positions; may alias P
 // when q == 0) and Wc (a' of the halo entries at their COMPACTED positions: the weights of bns_spmm_compact_f32)
@@ -522,71 +249,6 @@ inline unsigned gat_grid(int64_t n) {
 
 }  // namespace
 
-extern "C" int bns_gat_forward_f32(const bns_graph_t *a_in, const bns_graph_t *a_out, const int32_t *cidx,
-                                   const int32_t *chunk_cnt, const int32_t *cpos, int64_t x_halo_base, const float *ft,
-                                   int64_t ldft, int32_t H, int32_t Fo, const float *el, const float *er, float slope,
-                                   float p_drop, uint64_t seed, uint64_t offset, const uint64_t *offset_dev, float *rst,
-                                   int64_t ldr, float *P_in, float *P_out, void *stream) {
-    GatArgs a{};
-    int rc = gat_fill(a, a_in, a_out, cidx, chunk_cnt, cpos, x_halo_base, "bns_gat_forward_f32");
-    if (rc) return rc;
-    BNS_REQUIRE(H >= 1 && H <= kGatMaxHeads && Fo > 0 && Fo % 4 == 0 && (int64_t)H * Fo <= 1024,
-                "bns_gat_forward_f32: need 1 <= heads <= 8, out_feats %% 4 == 0, heads * out_feats <= 1024");
-    if (a.g.n_rows == 0) return BNS_OK;
-    BNS_REQUIRE(ft && el && er && rst && P_in && (a.g.cidx == nullptr || P_out), "bns_gat_forward_f32: NULL pointer");
-    BNS_REQUIRE(ldft % 4 == 0 && ldr % 4 == 0 && ldft >= H * Fo && ldr >= H * Fo &&
-                    ((reinterpret_cast<uintptr_t>(ft) | reinterpret_cast<uintptr_t>(rst)) & 15u) == 0,
-                "bns_gat_forward_f32: 16-byte aligned rows required");
-    BNS_REQUIRE(p_drop >= 0.f && p_drop < 1.f, "bns_gat_forward_f32: p must be in [0, 1)");
-    a.ft = ft; a.ldft = ldft; a.H = H; a.Fo = Fo; a.el = el; a.er = er; a.slope = slope; a.p_drop = p_drop;
-    a.keep_scale = 1.f / (1.f - p_drop); a.seed = seed; a.offset = offset; a.offset_dev = offset_dev;
-    a.rst = rst; a.ldr = ldr; a.P_in = P_in; a.P_out = P_out;
-    const int nv = (H * Fo + 127) / 128;
-    const unsigned grid = gat_grid(a.g.n_rows);
-    cudaStream_t st = as_stream(stream);
-    if (nv <= 1) gat_fwd_kernel<1><<<grid, kThreads, 0, st>>>(a, a_in->nnz);
-    else if (nv == 2) gat_fwd_kernel<2><<<grid, kThreads, 0, st>>>(a, a_in->nnz);
-    else if (nv <= 4) gat_fwd_kernel<4><<<grid, kThreads, 0, st>>>(a, a_in->nnz);
-    else gat_fwd_kernel<8><<<grid, kThreads, 0, st>>>(a, a_in->nnz);
-    ++g_launches;
-    BNS_CUDA(cudaGetLastError());
-    return BNS_OK;
-}
-
-extern "C" int bns_gat_backward_f32(const bns_graph_t *a_in, const bns_graph_t *a_out, const int32_t *cidx,
-                                    const int32_t *chunk_cnt, const int32_t *cpos, int64_t x_halo_base, const float *ft,
-                                    int64_t ldft, int32_t H, int32_t Fo, const float *el, const float *er, float slope,
-                                    float p_drop, uint64_t seed, uint64_t offset, const uint64_t *offset_dev,
-                                    const float *d_rst, int64_t ldd, const float *P_in, const float *P_out, float *dE_in,
-                                    float *dE_out, float *A_in, float *A_out, float *d_er, void *stream) {
-    GatArgs a{};
-    int rc = gat_fill(a, a_in, a_out, cidx, chunk_cnt, cpos, x_halo_base, "bns_gat_backward_f32");
-    if (rc) return rc;
-    BNS_REQUIRE(H >= 1 && H <= kGatMaxHeads && Fo > 0 && Fo % 4 == 0 && (int64_t)H * Fo <= 1024,
-                "bns_gat_backward_f32: need 1 <= heads <= 8, out_feats %% 4 == 0, heads * out_feats <= 1024");
-    if (a.g.n_rows == 0) return BNS_OK;
-    BNS_REQUIRE(ft && el && er && d_rst && P_in && dE_in && d_er && (a.g.cidx == nullptr || (P_out && dE_out)),
-                "bns_gat_backward_f32: NULL pointer");
-    BNS_REQUIRE((A_in == nullptr) == (A_out == nullptr) || a.g.cidx == nullptr, "bns_gat_backward_f32: A_in and A_out go together");
-    BNS_REQUIRE(ldft % 4 == 0 && ldd % 4 == 0 && ldft >= H * Fo && ldd >= H * Fo &&
-                    ((reinterpret_cast<uintptr_t>(ft) | reinterpret_cast<uintptr_t>(d_rst)) & 15u) == 0,
-                "bns_gat_backward_f32: 16-byte aligned rows required");
-    a.ft = ft; a.ldft = ldft; a.H = H; a.Fo = Fo; a.el = el; a.er = er; a.slope = slope; a.p_drop = p_drop;
-    a.keep_scale = 1.f / (1.f - p_drop); a.seed = seed; a.offset = offset; a.offset_dev = offset_dev;
-    a.d_rst = d_rst; a.ldd = ldd; a.P_in = const_cast<float *>(P_in); a.P_out = const_cast<float *>(P_out);
-    a.dE_in = dE_in; a.dE_out = dE_out; a.A_in = A_in; a.A_out = A_out; a.d_er = d_er;
-    const int nv = (H * Fo + 127) / 128;
-    const unsigned grid = gat_grid(a.g.n_rows);
-    cudaStream_t st = as_stream(stream);
-    if (nv <= 1) gat_bwd_kernel<1><<<grid, kThreads, 0, st>>>(a, a_in->nnz);
-    else if (nv == 2) gat_bwd_kernel<2><<<grid, kThreads, 0, st>>>(a, a_in->nnz);
-    else if (nv <= 4) gat_bwd_kernel<4><<<grid, kThreads, 0, st>>>(a, a_in->nnz);
-    else gat_bwd_kernel<8><<<grid, kThreads, 0, st>>>(a, a_in->nnz);
-    ++g_launches;
-    BNS_CUDA(cudaGetLastError());
-    return BNS_OK;
-}
-
 extern "C" int bns_gat_scores_f32(const bns_graph_t *a_in, const bns_graph_t *a_out, const int32_t *cidx, const int32_t *chunk_cnt,
                                   const int32_t *cpos, int64_t x_halo_base, int32_t H, const float *el, const float *er,
                                   float slope, float p_drop, uint64_t seed, uint64_t offset, const uint64_t *offset_dev,
@@ -599,7 +261,7 @@ extern "C" int bns_gat_scores_f32(const bns_graph_t *a_in, const bns_graph_t *a_
     BNS_REQUIRE(el && er && P_in && (a.g.cidx == nullptr || (P_out && W_out_compact)), "bns_gat_scores_f32: NULL pointer");
     BNS_REQUIRE(p_drop >= 0.f && p_drop < 1.f, "bns_gat_scores_f32: p must be in [0, 1)");
     BNS_REQUIRE(p_drop == 0.f || (W_in && (a.g.cidx == nullptr || W_out)), "bns_gat_scores_f32: dropout needs W_in / W_out");
-    a.H = H; a.Fo = 4; a.el = el; a.er = er; a.slope = slope; a.p_drop = p_drop; a.keep_scale = 1.f / (1.f - p_drop);
+    a.H = H; a.el = el; a.er = er; a.slope = slope; a.p_drop = p_drop; a.keep_scale = 1.f / (1.f - p_drop);
     a.seed = seed; a.offset = offset; a.offset_dev = offset_dev; a.P_in = P_in; a.P_out = P_out;
     int64_t want = (a.g.n_rows + kWarps - 1) / kWarps, cap = (int64_t)sm_count() * 8;
     gat_scores_kernel<<<(unsigned)(want < cap ? want : cap), kThreads, 0, as_stream(stream)>>>(a, a_in->nnz, W_in, W_out, W_out_compact);
@@ -619,7 +281,7 @@ extern "C" int bns_gat_softmax_bwd_f32(const bns_graph_t *a_in, const bns_graph_
     BNS_REQUIRE(H >= 1 && H <= kGatMaxHeads, "bns_gat_softmax_bwd_f32: 1 <= heads <= 8");
     if (a.g.n_rows == 0) return BNS_OK;
     BNS_REQUIRE(el && er && P_in && dE_in && d_er && (a.g.cidx == nullptr || (P_out && dE_out)), "bns_gat_softmax_bwd_f32: NULL pointer");
-    a.H = H; a.Fo = 4; a.el = el; a.er = er; a.slope = slope; a.p_drop = p_drop; a.keep_scale = 1.f / (1.f - p_drop);
+    a.H = H; a.el = el; a.er = er; a.slope = slope; a.p_drop = p_drop; a.keep_scale = 1.f / (1.f - p_drop);
     a.seed = seed; a.offset = offset; a.offset_dev = offset_dev;
     a.P_in = const_cast<float *>(P_in); a.P_out = const_cast<float *>(P_out); a.dE_in = dE_in; a.dE_out = dE_out; a.d_er = d_er;
     int64_t want = (a.g.n_rows + kWarps - 1) / kWarps, cap = (int64_t)sm_count() * 8;

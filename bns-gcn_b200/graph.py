@@ -12,8 +12,6 @@ from __future__ import annotations
 
 from typing import Dict, Optional
 
-import os
-
 import torch
 
 from . import ops
@@ -238,9 +236,7 @@ class GatAttention(torch.autograd.Function):
 
     Stages (include/bnsgcn.h): ``bns_gat_scores_f32`` (scalars: probabilities + dropped attention per entry) ->
     ``bns_spmm_weighted_f32`` / ``bns_spmm_compact_f32`` per head; backward ``bns_sddmm_dot_f32`` ->
-    ``bns_gat_softmax_bwd_f32`` -> ``bns_gat_colsum_f32`` -> ``bns_spmm_weighted_f32`` on the transposes.  The one-launch
-    row walks ``bns_gat_forward_f32`` / ``bns_gat_backward_f32`` compute the same thing (``BNS_GAT_ROWWALK=1``; the
-    tests run both) but are a latency chain per row on low-degree graphs: profiles/gat_r02.md."""
+    ``bns_gat_softmax_bwd_f32`` -> ``bns_gat_colsum_f32`` -> ``bns_spmm_weighted_f32`` on the transposes."""
 
     @staticmethod
     def forward(ctx, ft, el, er, g: PartitionGraph, H: int, Fo: int, slope: float, p: float, seed: int):
@@ -258,27 +254,21 @@ class GatAttention(torch.autograd.Function):
                 None if c is None else c.chunk_cnt.data_ptr(), None if c is None else c.cpos.data_ptr(), n_in)
         tail = (H, el.data_ptr(), er.data_ptr(), float(slope), float(p), seed & (2 ** 64 - 1), off & (2 ** 64 - 1),
                 ops._ptr(off_dev))
-        rowwalk = os.environ.get("BNS_GAT_ROWWALK", "0") == "1"
         st = torch.cuda.current_stream(dev).cuda_stream
         w_in = w_out = None
-        if rowwalk:
-            with torch.cuda.device(dev):
-                check(lib.bns_gat_forward_f32(*head, ft.data_ptr(), ft.stride(0), H, Fo, *tail[1:], rst.data_ptr(),
-                                              rst.stride(0), p_in.data_ptr(), ops._ptr(p_out), st), "bns_gat_forward_f32")
-        else:
-            if p > 0:
-                w_in = torch.empty_like(p_in)
-                w_out = torch.empty_like(p_out) if p_out is not None else None
-            wc = torch.empty_like(p_out) if p_out is not None else None          # halo attention, compacted positions
-            with torch.cuda.device(dev):
-                check(lib.bns_gat_scores_f32(*head, *tail, p_in.data_ptr(), ops._ptr(p_out), ops._ptr(w_in), ops._ptr(w_out),
-                                             ops._ptr(wc), st), "bns_gat_scores_f32")
-            for h in range(H):
-                cols = slice(h * Fo, (h + 1) * Fo)
-                ops.spmm_weighted(g.a_in, ft[:n_in, cols], rst[:, cols], p_in if w_in is None else w_in, h)
-                if c is not None:
-                    ops.spmm_compact(c, ft[n_in:, cols], rst[:, cols], accumulate=True, weights=wc, head=h)
-        ctx.g, ctx.c, ctx.head, ctx.tail, ctx.cfg, ctx.rowwalk = g, c, head, tail, (H, Fo, float(p)), rowwalk
+        if p > 0:
+            w_in = torch.empty_like(p_in)
+            w_out = torch.empty_like(p_out) if p_out is not None else None
+        wc = torch.empty_like(p_out) if p_out is not None else None          # halo attention, compacted positions
+        with torch.cuda.device(dev):
+            check(lib.bns_gat_scores_f32(*head, *tail, p_in.data_ptr(), ops._ptr(p_out), ops._ptr(w_in), ops._ptr(w_out),
+                                         ops._ptr(wc), st), "bns_gat_scores_f32")
+        for h in range(H):
+            cols = slice(h * Fo, (h + 1) * Fo)
+            ops.spmm_weighted(g.a_in, ft[:n_in, cols], rst[:, cols], p_in if w_in is None else w_in, h)
+            if c is not None:
+                ops.spmm_compact(c, ft[n_in:, cols], rst[:, cols], accumulate=True, weights=wc, head=h)
+        ctx.g, ctx.c, ctx.head, ctx.tail, ctx.cfg = g, c, head, tail, (H, Fo, float(p))
         saved = [ft, el, er, p_in] + ([p_out] if p_out is not None else [])
         if w_in is not None:
             saved += [w_in] + ([w_out] if w_out is not None else [])
@@ -299,28 +289,18 @@ class GatAttention(torch.autograd.Function):
         de_out = torch.empty_like(p_out) if p_out is not None else None
         d_er = torch.empty(n_in, H, dtype=torch.float32, device=dev)
         st = torch.cuda.current_stream(dev).cuda_stream
-        if ctx.rowwalk:
-            a_in = torch.empty_like(p_in) if p > 0 else None
-            a_out = torch.empty_like(p_out) if (p > 0 and p_out is not None) else None
-            with torch.cuda.device(dev):
-                check(lib.bns_gat_backward_f32(*ctx.head, ft.data_ptr(), ft.stride(0), H, Fo, *ctx.tail[1:], d_rst.data_ptr(),
-                                               d_rst.stride(0), p_in.data_ptr(), ops._ptr(p_out), de_in.data_ptr(),
-                                               ops._ptr(de_out), ops._ptr(a_in), ops._ptr(a_out), d_er.data_ptr(), st),
-                      "bns_gat_backward_f32")
-            w_in, w_out = (a_in, a_out) if p > 0 else (p_in, p_out)
-        else:
-            w_in, w_out = p_in, p_out
-            if ctx.n_w:
-                w_in = rest.pop(0)
-                w_out = rest.pop(0) if ctx.n_w == 2 else None
-            for h in range(H):                                 # d a'_uv = <d rst_v, ft_u> (0 for an unsampled halo node)
-                cols = slice(h * Fo, (h + 1) * Fo)
-                ops.sddmm_dot(g.a_in, d_rst[:, cols], ft[:n_in, cols], out=de_in[:, h])
-                if c is not None:
-                    ops.sddmm_dot(g.a_out, d_rst[:, cols], ft[n_in:, cols], col_map=g.slot, n_direct=0, out=de_out[:, h])
-            with torch.cuda.device(dev):
-                check(lib.bns_gat_softmax_bwd_f32(*ctx.head, *ctx.tail, p_in.data_ptr(), ops._ptr(p_out), de_in.data_ptr(),
-                                                  ops._ptr(de_out), d_er.data_ptr(), st), "bns_gat_softmax_bwd_f32")
+        w_in, w_out = p_in, p_out
+        if ctx.n_w:
+            w_in = rest.pop(0)
+            w_out = rest.pop(0) if ctx.n_w == 2 else None
+        for h in range(H):                                 # d a'_uv = <d rst_v, ft_u> (0 for an unsampled halo node)
+            cols = slice(h * Fo, (h + 1) * Fo)
+            ops.sddmm_dot(g.a_in, d_rst[:, cols], ft[:n_in, cols], out=de_in[:, h])
+            if c is not None:
+                ops.sddmm_dot(g.a_out, d_rst[:, cols], ft[n_in:, cols], col_map=g.slot, n_direct=0, out=de_out[:, h])
+        with torch.cuda.device(dev):
+            check(lib.bns_gat_softmax_bwd_f32(*ctx.head, *ctx.tail, p_in.data_ptr(), ops._ptr(p_out), de_in.data_ptr(),
+                                              ops._ptr(de_out), d_er.data_ptr(), st), "bns_gat_softmax_bwd_f32")
         with torch.cuda.device(dev):
             d_el = torch.empty(n_u, H, dtype=torch.float32, device=dev)
             check(lib.bns_gat_colsum_f32(g.a_in_t._h, de_in.data_ptr(), H, None, 0, d_el.data_ptr(), st),

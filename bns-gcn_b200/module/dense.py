@@ -6,135 +6,26 @@ pass would miss the 1e-4 parity bar (10-bit mantissa).  ``linear()`` therefore u
 scheme: split every f32 operand into ``hi = tf32(x)`` and ``lo = x - hi`` (exact in f32) and accumulate
 ``hi*hi + hi*lo + lo*hi`` on the tensor cores with f32 accumulation; the dropped ``lo*lo`` term is 2^-22 relative.
 
-``MODE`` (env BNS_DENSE): "tc" (default) -- the hand-written tcgen05 kernels of csrc/dense_tc.cuh: 3xTF32 with the
-operand split fused into the TMA -> shared memory -> TMEM pipeline (forward, input gradient, split-K weight gradient);
-operands whose rows are not 16-byte multiples fall back to fp32 cuBLAS | "fp32" (cuBLAS SIMT, the literal reference
-precision) | "auto" (library-composed 3xtf32 where K >= 512) | "3xtf32" | "bf16x3".
+It runs in the hand-written tcgen05 kernels of csrc/dense_tc.cuh, with the operand split fused into the TMA -> shared
+memory -> TMEM pipeline (forward, input gradient, split-K weight gradient).  Operands whose rows are not 16-byte
+multiples go to fp32 cuBLAS, the literal reference precision.
 B200, M=232,965 K=1204 N=256 (tools/check_dense_tc.py perf): fp32 cuBLAS 2.37 ms fwd / 3.15 ms dW; tc 0.95 / 0.97 ms
 with max error 2.7e-6 / 3.5e-6 of max|C| against f64 (cuBLAS fp32: 1.9e-6 / 1.5e-6).  History: the library-composed
 3xtf32 (three cuBLAS TF32 GEMMs + a split pass) was slower than fp32 cuBLAS except at K >= 512, bf16x3 always slower
-(profiles/bench_n1_r01_*_negative_result.json).
+(profiles/bench_n1_r01_*_negative_result.json); both were removed, which is why there is one mode.
 """
-import os
+import threading
 
 import torch
 import torch.nn.functional as F
-
-import threading
 
 # torch.backends.cuda.matmul.allow_tf32 is process-global and read at enqueue time.  Ranks that are threads of one
 # process (tests, smoke) must not see each other's setting: every GEMM of this module is enqueued under this lock,
 # fp32 ones included (forward AND backward -- hence the custom fp32 Function below instead of F.linear).
 _GEMM_LOCK = threading.RLock()
 
-MODE = os.environ.get("BNS_DENSE", "tc")
 # bench.py sets this to a list to collect (start_event, end_event, useful_flops, algorithmic_bytes) per tcgen05 GEMM
 PROFILE = None
-MIN_K_3X = 512       # "auto": 3xTF32 only where the GEMM is big enough to repay the split pass (layer 0: K = 2 * n_feat)
-
-
-def _split(t: torch.Tensor):
-    """hi = t rounded to TF32 (10 explicit mantissa bits, round-to-nearest on the 13 dropped bits), lo = t - hi.
-    One fused pass (``bns_split_tf32_f32``) on CUDA; torch ops elsewhere (CPU checks)."""
-    t = t.contiguous()
-    if t.is_cuda and t.numel() % 4 == 0:
-        from .._lib import check, lib
-        hi, lo = torch.empty_like(t), torch.empty_like(t)
-        with torch.cuda.device(t.device):
-            check(lib.bns_split_tf32_f32(t.data_ptr(), t.numel(), hi.data_ptr(), lo.data_ptr(),
-                                         torch.cuda.current_stream().cuda_stream), "bns_split_tf32_f32")
-        return hi, lo
-    bits = t.view(torch.int32)
-    hi = ((bits + 0x1000) & -0x2000).view(torch.float32)
-    return hi, t - hi
-
-
-def _mm3(a2, b2, trans_a=False, trans_b=False) -> torch.Tensor:
-    """op(a) @ op(b) with 3xTF32 error compensation; ``a2`` / ``b2`` are (hi, lo) pairs."""
-    (ah, al), (bh, bl) = a2, b2
-    if trans_a:
-        ah, al = ah.t(), al.t()
-    if trans_b:
-        bh, bl = bh.t(), bl.t()
-    with _GEMM_LOCK:
-        prev = torch.backends.cuda.matmul.allow_tf32
-        torch.backends.cuda.matmul.allow_tf32 = True
-        try:
-            out = torch.mm(al, bh)          # small terms first, then the dominant one: better rounding
-            out.addmm_(ah, bl)
-            out.addmm_(ah, bh)
-        finally:
-            torch.backends.cuda.matmul.allow_tf32 = prev
-    return out
-
-
-class _Linear3x(torch.autograd.Function):
-
-    @staticmethod
-    def forward(ctx, x, weight, bias):
-        x2, w2 = _split(x), _split(weight)
-        ctx.x2, ctx.w2, ctx.has_bias = x2, w2, bias is not None
-        y = _mm3(x2, w2, trans_b=True)
-        if bias is not None:
-            y += bias
-        return y
-
-    @staticmethod
-    def backward(ctx, dy):
-        d2 = _split(dy)
-        dx = _mm3(d2, ctx.w2) if ctx.needs_input_grad[0] else None
-        dw = _mm3(d2, ctx.x2, trans_a=True) if ctx.needs_input_grad[1] else None
-        db = dy.sum(0) if ctx.has_bias and ctx.needs_input_grad[2] else None
-        ctx.x2 = ctx.w2 = None
-        return dx, dw, db
-
-
-# ---- bf16x3: x = b0 + b1 + b2 (24 mantissa bits), six bf16 tensor-core GEMMs, f32 accumulation ----------------------
-_PAIRS = ((2, 0), (0, 2), (1, 1), (1, 0), (0, 1), (0, 0))          # small terms first
-
-
-def _split3(t: torch.Tensor):
-    from .._lib import check, lib
-    t = t.contiguous()
-    n = t.numel()
-    if n % 4:
-        raise RuntimeError("bf16x3 split needs a multiple of 4 elements")
-    outs = [torch.empty(t.shape, dtype=torch.bfloat16, device=t.device) for _ in range(3)]
-    with torch.cuda.device(t.device):
-        check(lib.bns_split_bf16x3_f32(t.data_ptr(), n, outs[0].data_ptr(), outs[1].data_ptr(), outs[2].data_ptr(),
-                                       torch.cuda.current_stream().cuda_stream), "bns_split_bf16x3_f32")
-    return outs
-
-
-def _mm6(a3, b3, trans_a=False, trans_b=False):
-    """sum over i + j <= 2 of  op(a_i) @ op(b_j)  in f32."""
-    acc = None
-    for i, j in _PAIRS:
-        a = a3[i].t() if trans_a else a3[i]
-        b = b3[j].t() if trans_b else b3[j]
-        acc = torch.mm(a, b, out_dtype=torch.float32) if acc is None else torch.addmm(acc, a, b, out_dtype=torch.float32)
-    return acc
-
-
-class _LinearBf16x3(torch.autograd.Function):
-
-    @staticmethod
-    def forward(ctx, x, weight, bias):
-        x3, w3 = _split3(x), _split3(weight)
-        ctx.x3, ctx.w3, ctx.has_bias = x3, w3, bias is not None
-        y = _mm6(x3, w3, trans_b=True)                      # [M,K] @ [N,K]^T
-        if bias is not None:
-            y += bias
-        return y
-
-    @staticmethod
-    def backward(ctx, dy):
-        d3 = _split3(dy)
-        dx = _mm6(d3, ctx.w3) if ctx.needs_input_grad[0] else None                # [M,N] @ [N,K]
-        dw = _mm6(d3, ctx.x3, trans_a=True) if ctx.needs_input_grad[1] else None  # [M,N]^T @ [M,K]
-        db = dy.sum(0) if ctx.has_bias and ctx.needs_input_grad[2] else None
-        ctx.x3 = ctx.w3 = None
-        return dx, dw, db
 
 
 class _LinearFp32(torch.autograd.Function):
@@ -157,7 +48,7 @@ class _LinearFp32(torch.autograd.Function):
         return dx, dw, db
 
 
-# ---- "tc": hand-written tcgen05 kernels (csrc/dense_tc.cuh), 3xTF32 with the split fused into the pipeline ---------
+# ---- hand-written tcgen05 kernels (csrc/dense_tc.cuh), 3xTF32 with the split fused into the pipeline --------------
 def _tc_operand(t: torch.Tensor) -> bool:
     return (t.is_cuda and t.dtype == torch.float32 and t.dim() == 2 and t.stride(1) == 1 and t.stride(0) % 4 == 0
             and t.stride(0) >= t.shape[1] and t.data_ptr() % 16 == 0 and t.shape[0] > 0 and t.shape[1] > 0)
@@ -278,7 +169,7 @@ class _LinearTc(torch.autograd.Function):
 
 def linear(x: torch.Tensor, weight: torch.Tensor, bias=None, addend=None) -> torch.Tensor:
     """Drop-in for ``F.linear`` on 2-D f32 CUDA inputs; ``addend`` ([M, >= out_features], extra columns ignored) is
-    added to the result -- inside the GEMM epilogue in "tc" mode (when it has exactly the padded output width)."""
+    added to the result -- inside the GEMM epilogue when it has exactly the padded output width."""
     n = weight.shape[0]
     if addend is not None:
         y = _linear(x, weight, bias, addend)
@@ -288,30 +179,21 @@ def linear(x: torch.Tensor, weight: torch.Tensor, bias=None, addend=None) -> tor
 
 def _linear(x, weight, bias, addend):
     """Returns None when ``addend`` was given but cannot be fused (the caller adds it)."""
-    ok = x.is_cuda and x.dtype == torch.float32 and x.dim() == 2
-    if MODE == "tc" and ok:
-        n = weight.shape[0]
-        pad = (-n) % 4
-        add_ok = addend is None or (_tc_operand(addend) and addend.shape[0] == x.shape[0] and addend.shape[1] == n + pad)
-        if pad == 0:
-            if add_ok and tc_eligible(x, weight, bias):
-                return _LinearTc.apply(x, weight, bias, addend)
-        elif add_ok and weight.dim() == 2 and weight.is_cuda and weight.dtype == torch.float32:
-            # e.g. 41 classes: run 44 output columns (zero rows of W) so that every row stays 16-byte aligned for TMA
-            # and slice; autograd pads dY / slices dW accordingly
-            w = F.pad(weight, (0, 0, 0, pad))
-            b = F.pad(bias, (0, pad)) if bias is not None else None
-            if tc_eligible(x, w, b):
-                return _LinearTc.apply(x, w, b, addend)[:, :n]
-        if addend is not None:
-            return None
-        return _LinearFp32.apply(x, weight, bias)        # shapes TMA cannot address (rows not 16-byte multiples)
+    if not (x.is_cuda and x.dtype == torch.float32 and x.dim() == 2):
+        return None if addend is not None else F.linear(x, weight, bias)
+    n = weight.shape[0]
+    pad = (-n) % 4
+    add_ok = addend is None or (_tc_operand(addend) and addend.shape[0] == x.shape[0] and addend.shape[1] == n + pad)
+    if pad == 0:
+        if add_ok and tc_eligible(x, weight, bias):
+            return _LinearTc.apply(x, weight, bias, addend)
+    elif add_ok and weight.dim() == 2 and weight.is_cuda and weight.dtype == torch.float32:
+        # e.g. 41 classes: run 44 output columns (zero rows of W) so that every row stays 16-byte aligned for TMA
+        # and slice; autograd pads dY / slices dW accordingly
+        w = F.pad(weight, (0, 0, 0, pad))
+        b = F.pad(bias, (0, pad)) if bias is not None else None
+        if tc_eligible(x, w, b):
+            return _LinearTc.apply(x, w, b, addend)[:, :n]
     if addend is not None:
         return None
-    if MODE == "bf16x3" and ok and x.numel() % 4 == 0 and weight.numel() % 4 == 0 and weight.shape[0] % 4 == 0:
-        return _LinearBf16x3.apply(x, weight, bias)
-    if ok and (MODE == "3xtf32" or (MODE == "auto" and x.shape[1] >= MIN_K_3X)):
-        return _Linear3x.apply(x, weight, bias)
-    if ok:
-        return _LinearFp32.apply(x, weight, bias)
-    return F.linear(x, weight, bias)
+    return _LinearFp32.apply(x, weight, bias)        # shapes TMA cannot address (rows not 16-byte multiples)

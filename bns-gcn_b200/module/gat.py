@@ -7,10 +7,10 @@ call the reference makes -- ``layer(g, (h_src, h_dst))`` on the bipartite ``_U -
     e_uv = leaky_relu(el_u + er_v)   a = attn_drop(edge_softmax(e))     rst_v = sum_u a_uv ft_u + bias
 
 Everything after ``fc`` runs as kernels of libbnsgcn.so (``graph.GatProjection``, ``graph.GatAttention``; feature
-dropout on the Philox kernel).  The op-by-op fallback (``BNS_GAT_FUSED=0`` or a per-head width that is not a multiple
-of 4) writes the per-entry score / softmax algebra as torch ops on ``[nnz, heads]`` vectors over the STATIC entry lists
-of the partition graph (an unsampled halo entry gets e = -inf, i.e. weight 0) around the weighted SpMM, its transpose
-and the SDDMM-dot of the attention gradient (``graph.WeightedAggregate``)."""
+dropout on the Philox kernel).  The op-by-op fallback (a per-head width that is not a multiple of 4) writes the
+per-entry score / softmax algebra as torch ops on ``[nnz, heads]`` vectors over the STATIC entry lists of the
+partition graph (an unsampled halo entry gets e = -inf, i.e. weight 0) around the weighted SpMM, its transpose and the
+SDDMM-dot of the attention gradient (``graph.WeightedAggregate``)."""
 import torch
 import torch.nn.functional as F
 from torch import nn
@@ -18,12 +18,6 @@ from torch import nn
 from .. import fused, ops
 from ..graph import GatAttention, GatProjection, PartitionGraph, WeightedAggregate, gat_entries
 from . import dense
-
-
-# the attention (u_add_v, leaky_relu, edge_softmax, attn_drop, u_mul_e + sum of DGL's GATConv) as kernels
-# (graph.GatAttention); False / per-head widths that are not multiples of 4: the op-by-op torch path below
-import os as _os
-FUSED_ATTENTION = _os.environ.get("BNS_GAT_FUSED", "1") != "0"
 
 
 class GATConv(nn.Module):
@@ -59,7 +53,9 @@ class GATConv(nn.Module):
         ready = getattr(feat[0], '_bns_ready', None)
         if ready is not None:          # every row of h_src is read below: wait for the overlapped exchange
             torch.cuda.current_stream(feat[0].device).wait_event(ready)
-        kernels = FUSED_ATTENTION and Fo % 4 == 0 and H <= 8 and H * Fo <= 1024 and \
+        # the attention (u_add_v, leaky_relu, edge_softmax, attn_drop, u_mul_e + sum of DGL's GATConv) as kernels
+        # (graph.GatAttention); per-head widths that are not multiples of 4: the op-by-op torch path below
+        kernels = Fo % 4 == 0 and H <= 8 and H * Fo <= 1024 and \
             (graph.a_out is None or (graph.compact is not None and graph.compact.cpos is not None))
         salt = ops.RNG["seed"] + 15485863 * (1 + getattr(self, "_layer_index", 0))
         pf = self.feat_drop.p if self.training else 0.0

@@ -334,11 +334,9 @@ class TrainState:
 
 def _fused_eligible(args, layer_size, dev) -> bool:
     """The fused training step (fused.py) covers the BASELINE configuration families: GraphSAGE / GCN, --use-pp, LayerNorm +
-    ReLU between the layers, no trailing linear layers, widths the 16-byte vector / TMA paths take.  BNS_FUSED=0 turns
-    it off (the op-by-op autograd path, kept for every other configuration, then runs here too)."""
-    import os
-    from .module import dense
-    if os.environ.get("BNS_FUSED", "1") == "0" or dense.MODE != "tc" or dev.type != "cuda":
+    ReLU between the layers, no trailing linear layers, widths the 16-byte vector / TMA paths take.  Every other
+    configuration runs the op-by-op autograd path."""
+    if dev.type != "cuda":
         return False
     if args.model not in ('graphsage', 'gcn') or not args.use_pp or args.n_linear != 0 or args.norm != 'layer':
         return False

@@ -36,7 +36,7 @@ extern "C" {
 #define BNS_E_WORKSPACE  (-3)   /* workspace too small */
 #define BNS_E_UNSUPPORTED (-4)
 
-#define BNS_ABI_VERSION 2
+#define BNS_ABI_VERSION 3
 
 typedef struct bns_graph bns_graph_t;   /* opaque: a static CSR matrix resident in HBM */
 typedef struct bns_p2p   bns_p2p_t;     /* opaque: peer-mapped exchange slabs of one rank */
@@ -107,16 +107,6 @@ int bns_spmm_sum_f32(const bns_graph_t *g,
                      int64_t x_rows /*rows of X that can be referenced (0 = n_cols); sizes the L2 blocking*/,
                      int32_t slab_hint /*0 = automatic; 256 | 128 | 64 | 32 forces the column-slab width*/,
                      int accumulate, void *ws, size_t ws_bytes, void *stream);
-
-/* ------------------------------------------------------------------------------------------------
- * K8 helper (dense layers): split n contiguous f32 values into three bf16 arrays with x = b0 + b1 + b2 exact to
- * 24 mantissa bits (round-to-nearest-even at each step).  Six bf16 tensor-core GEMMs b_i * w_j (i + j <= 2) with f32
- * accumulation then reproduce the f32 product to ~2^-23 (module/dense.py, mode "bf16x3").  n % 4 == 0.
- * ----------------------------------------------------------------------------------------------*/
-int bns_split_bf16x3_f32(const float *x, int64_t n, void *out0 /*bf16 [n]*/, void *out1, void *out2, void *stream);
-/* Same idea with TF32 (module/dense.py "3xtf32"): hi = x rounded to 10 mantissa bits, lo = x - hi (exact);
- * hi*hi + hi*lo + lo*hi in three TF32 tensor-core GEMMs with f32 accumulation is f32-accurate to ~2^-21. */
-int bns_split_tf32_f32(const float *x, int64_t n, float *hi, float *lo, void *stream);
 
 /* ------------------------------------------------------------------------------------------------
  * K8: the dense layers themselves.  Replaces, for 2-D f32 operands,
@@ -311,35 +301,24 @@ int bns_spmm_compact_f32(const bns_graph_t *g, const int32_t *cidx, const float 
                          void *stream);
 
 /* ------------------------------------------------------------------------------------------------
- * K10 fused: the attention of dgl.nn.GATConv (module/model.py:96-132; DGL 0.9 python/dgl/nn/pytorch/conv/gatconv.py):
+ * K10 staged: the attention of dgl.nn.GATConv (module/model.py:96-132; DGL 0.9 python/dgl/nn/pytorch/conv/gatconv.py):
  *     e_uv = leaky_relu(el_u + er_v);  p = edge_softmax(e) over each destination's in-entries;  a = attn_drop(p);
- *     rst_v = sum_u a_uv ft_u                     for all `heads` at once, one warp per destination row.
+ *     rst_v = sum_u a_uv ft_u                     for all `heads` at once.
  * The entries of row v are those of a_in followed by the SAMPLED ones of a_out (cidx / chunk_cnt / cpos from
  * bns_graph_compact_cols with col_map = slot, n_direct = 0; halo source k reads ft row x_halo_base + k).
- *   ft [n_u, heads * out_feats] (head-major columns), el [n_u, heads], er [n_in, heads]; out_feats % 4 == 0,
- *   heads <= 8, heads * out_feats <= 1024.  P_in [nnz(a_in), heads] / P_out [nnz(a_out), heads]: the probabilities,
- *   stored at the ORIGINAL entry positions, kept for the backward.  Dropout: Philox4x32-10(counter = (entry, head),
- *   key = seed, offset [+ *offset_dev]), regenerated in backward.
- * bns_gat_backward_f32: d e per entry into dE_in / dE_out (same layout as P), d er [n_in, heads], and the dropped
- *   attention a = p * mask / (1 - q) into A_in / A_out (NULL when q == 0: then a = p).
- * bns_gat_colsum_f32 (on a_in_t, then on a_out_t with row_map = slot): d el_u = sum over column u of d e.
- * bns_spmm_weighted_f32: d ft = A^T d rst, one head per call, the attention read through the transpose's permutation.
+ *   el [n_u, heads], er [n_in, heads], heads <= 8.  P_in [nnz(a_in), heads] / P_out [nnz(a_out), heads]: the
+ *   probabilities, stored at the ORIGINAL entry positions, kept for the backward.  Dropout: Philox4x32-10(counter =
+ *   (entry, head), key = seed, offset [+ *offset_dev]), regenerated in backward.
+ * Each stage keeps thousands of independent gathers in flight:
+ *   forward   bns_gat_scores_f32 -- scalars only, one warp per destination row: P and the dropped attention
+ *             W = p * mask / (1 - q) at the original positions, W_out_compact at the compacted positions -- then
+ *             rst = W ft by bns_spmm_weighted_f32 / bns_spmm_compact_f32, one head per call;
+ *   backward  bns_sddmm_dot_f32 writes d a' = <d rst_v, ft_u> into dE_in / dE_out (same layout as P);
+ *             bns_gat_softmax_bwd_f32 turns it into d e in place and writes d er [n_in, heads];
+ *             bns_gat_colsum_f32 (on a_in_t, then on a_out_t with row_map = slot): d el_u = sum over column u of d e;
+ *             bns_spmm_weighted_f32: d ft = W^T d rst, one head per call, the attention read through the transpose's
+ *             permutation.
  * ----------------------------------------------------------------------------------------------*/
-int bns_gat_forward_f32(const bns_graph_t *a_in, const bns_graph_t *a_out /*or NULL*/, const int32_t *cidx,
-                        const int32_t *chunk_cnt, const int32_t *cpos, int64_t x_halo_base, const float *ft, int64_t ldft,
-                        int32_t heads, int32_t out_feats, const float *el, const float *er, float negative_slope, float p_drop,
-                        uint64_t seed, uint64_t offset, const uint64_t *offset_dev, float *rst, int64_t ldr, float *P_in,
-                        float *P_out, void *stream);
-int bns_gat_backward_f32(const bns_graph_t *a_in, const bns_graph_t *a_out, const int32_t *cidx, const int32_t *chunk_cnt,
-                         const int32_t *cpos, int64_t x_halo_base, const float *ft, int64_t ldft, int32_t heads,
-                         int32_t out_feats, const float *el, const float *er, float negative_slope, float p_drop, uint64_t seed,
-                         uint64_t offset, const uint64_t *offset_dev, const float *d_rst, int64_t ldd, const float *P_in,
-                         const float *P_out, float *dE_in, float *dE_out, float *A_in, float *A_out, float *d_er, void *stream);
-/* The same algebra decomposed (what graph.GatAttention runs: each stage has thousands of independent gathers in flight,
- * where one fused row walk is a latency chain per row): bns_gat_scores_f32 -- scalars only: probabilities P and dropped
- * attention W at the original positions, W_out_compact at the compacted positions -- then bns_spmm_weighted_f32 /
- * bns_spmm_compact_f32 per head; backward: bns_sddmm_dot_f32 into dE, bns_gat_softmax_bwd_f32 (dE: d a' -> d e in
- * place, d er), bns_gat_colsum_f32, bns_spmm_weighted_f32 through the permutation. */
 int bns_gat_scores_f32(const bns_graph_t *a_in, const bns_graph_t *a_out, const int32_t *cidx, const int32_t *chunk_cnt,
                        const int32_t *cpos, int64_t x_halo_base, int32_t heads, const float *el, const float *er,
                        float negative_slope, float p_drop, uint64_t seed, uint64_t offset, const uint64_t *offset_dev,

@@ -56,15 +56,18 @@ def test_strided_rows_and_onehot_are_exact(dense):
 
 
 def test_linear_autograd_matches_f64_and_pads_odd_widths(dense):
-    """`linear()` in tc mode: forward, dX, dW, db against f64 -- including 41 output columns (padded to 44)."""
-    assert dense.MODE == "tc"
+    """`linear()` runs on the tcgen05 kernels (not the cuBLAS fallback): forward, dX, dW, db against f64 -- including
+    41 output columns (padded to 44)."""
+    from bns_gcn_b200._lib import lib
     for n_out in (64, 41):
         g = torch.Generator().manual_seed(n_out)
         x = torch.randn(3000, 256, generator=g).cuda().requires_grad_()
         w = (torch.randn(n_out, 256, generator=g) / 16).cuda().requires_grad_()
         b = torch.randn(n_out, generator=g).cuda().requires_grad_()
         dy = torch.randn(3000, n_out, generator=g).cuda()
+        launches = lib.bns_launch_count()
         y = dense.linear(x, w, b)
+        assert lib.bns_launch_count() > launches, "linear() did not reach the tcgen05 kernels"
         assert y.shape == (3000, n_out)
         y.backward(dy)
         xd, wd, bd, dyd = x.detach().double(), w.detach().double(), b.detach().double(), dy.double()
